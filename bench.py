@@ -5,6 +5,11 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path, headline workload
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's CPU path, same workload
     python bench.py --workload {cdu_closed_loop,horizon_sweep,cstr_qp_1m,nn_10m} ...
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's results
+
+--dump-outputs DIR writes what the timed path returned in its last timed step (rank 0) as DIR/<name>.npy, float64,
+64 MB at most: above that, the same seeded sample of batch rows of every array.  The inputs are seeded, so two
+builds run with the same arguments can be compared file by file (bench_outputs/ is ignored by git).
 
 Workloads (BASELINE.json configs[...]):
   cdu_closed_loop [2]  default, the headline.  The crude-distillation linear MPC of the reference (252 states,
@@ -47,6 +52,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 KKT_TOL = 1e-8
+DUMP_BYTES = 64_000_000
 WORKLOADS = {
     "cdu_closed_loop": ("cdu_closed_loop_sim_steps_per_s", "sim-steps/s"),
     "horizon_sweep": ("cdu_closed_loop_sim_steps_per_s", "sim-steps/s"),
@@ -65,6 +71,24 @@ def _peaks():
         with open(path) as f:
             return json.load(f), "measured (MEASURED_PEAKS.json)"
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0}, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(dirname, arrays, seed=0):
+    """--dump-outputs: every array (batch axis first; CUDA tensor or NumPy) -> dirname/<name>.npy in float64.  Above
+    DUMP_BYTES in all, every array keeps the same seeded, sorted sample of batch rows."""
+    rows = next(iter(arrays.values())).shape[0]
+    assert all(a.shape[0] == rows for a in arrays.values()), {k: tuple(a.shape) for k, a in arrays.items()}
+    row_bytes = sum(8 * int(np.prod(a.shape[1:])) for a in arrays.values())
+    keep = min(rows, (DUMP_BYTES - 4096 * len(arrays)) // row_bytes)       # 4 kB per file for the .npy header
+    idx = np.arange(rows) if keep == rows else np.sort(np.random.default_rng(seed).choice(rows, keep, replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if isinstance(a, np.ndarray):
+            a = a[idx]
+        else:                                    # gather the sample on the device, copy only that
+            import torch
+            a = a.index_select(0, torch.as_tensor(idx, device=a.device)).cpu().numpy()
+        np.save(os.path.join(dirname, name + ".npy"), a.astype(np.float64))
 
 
 class ClockSampler:
@@ -476,6 +500,9 @@ def run_cdu(args):
     kkt_max, it_sum, it_max = float(kkt_acc), int(it_sum), int(it_acc)
     clocks = clk.summary()
     value = world * B * Ts * K / (ms_dev * 1e-3)
+    if args.dump_outputs and rank == 0:          # before the profiled pass reuses the result buffers
+        dump_outputs(args.dump_outputs, {k: r[k] for k in ("x", "uprev", "xs", "us", "u", "iters", "kkt",
+                                                           "x_final", "uprev_final")})
 
     # ---- profiled pass: the same kind of steps with the library's CUDA-event spans switched on ----
     Kp = max(1, min(K, args.prof_steps))
@@ -755,6 +782,8 @@ def run_cstr_qp(args):
     active = float(((Us == LB[:, None, :]) | (Us == UB[:, None, :])).any(dim=2).any(dim=1).double().mean())
     if kkt_max > KKT_TOL or info["maxiter_hit"]:
         raise SystemExit(f"bench.py: timed solves missed the tolerance (kkt {kkt_max:.2e}); number rejected")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"U": U, "cost": info["cost"], "kkt": info["kkt"], "iters": info["iters"]})
     # profiled pass
     _lib.prof_enable(True)
     _lib.prof_read(reset=True)
@@ -873,6 +902,8 @@ def run_nn(args):
     ms_dev = ctx.maxrank(ev0.elapsed_time(ev1))
     launches = L.nnmpc_launch_count() - launches0
     value = world * B * K / (ms_dev * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"u": out})
     # validity: a sample of the timed outputs against the NumPy restatement (tolerance of the north star: 1e-5)
     pick = torch.randint(0, B, (512,), device=dev, generator=g)
     ins = [t[pick].cpu().numpy() for t in (x, up, xs, us)]
@@ -1054,7 +1085,14 @@ def main():
     ap.add_argument("--r-weight", type=float, default=None, help="conditioning study: R = r I (reference tuning: 0.1)")
     ap.add_argument("--max-iter", type=int, default=None,
                     help="per-QP iteration cap (a hit rejects the number); default 3000 (CDU closed loop) / 20000 (cold CSTR QPs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (float64, seeded row sample, "
+                         "64 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of this repository's CUDA path, not of --impl reference")
     if args.traj is None:
         args.traj = 16384 if args.workload == "horizon_sweep" else 65536
     if args.max_iter is None:

@@ -58,6 +58,25 @@ def test_cpu_pool_steps_are_timed_closed_loop_steps():
         pool.close()
 
 
+def test_dump_outputs_writes_float64_within_budget_and_samples_the_same_rows(tmp_path, monkeypatch):
+    rng = np.random.default_rng(5)
+    small = {"u": rng.standard_normal((7, 3)), "iters": np.arange(7, dtype=np.int32)}
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    for k, v in small.items():
+        back = np.load(tmp_path / "small" / f"{k}.npy")
+        assert back.dtype == np.float64 and np.array_equal(back, v)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 64_000)
+    big = {"x": np.arange(5000 * 4 * 3, dtype=np.float64).reshape(5000, 4, 3), "kkt": np.arange(5000.0)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big)
+    files = sorted((tmp_path / "a").iterdir())
+    assert sum(f.stat().st_size for f in files) <= 64_000
+    x, kkt = np.load(tmp_path / "a" / "x.npy"), np.load(tmp_path / "a" / "kkt.npy")
+    rows = kkt.astype(int)
+    assert 0 < len(rows) < 5000 and np.all(np.diff(rows) > 0) and np.array_equal(x, big["x"][rows])
+    assert all(np.array_equal(np.load(f), np.load(tmp_path / "b" / f.name)) for f in files)
+
+
 def test_scenarios_are_contiguous_chunks_of_one_prbs_signal():
     p, sp, ds = bench._scenarios(5, 400, seed=3)
     assert sp.shape == (5, 400, p.Ny) and ds.shape == (5, 400, p.Nd)
