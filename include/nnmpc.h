@@ -280,6 +280,20 @@ int nnmpc_lp_gemm_test(int M, int N, int K, const double* A, const double* Bt, d
  * operands, exact INT32 accumulation, 36 INT8 products), C[M x N] = A[M x K] Bt[N x K]^T; dense row-major FP64
  * device matrices, K <= 32768. */
 int nnmpc_oz_gemm_test(int M, int N, int K, const double* A, const double* Bt, double* C, void* stream);
+/* nnmpc_exact_apply_test: the exact operator applies of the closed-loop engine, called as the engine calls them.
+ *   kind 0: anchor  X[r] = Op A[r] - C[r]
+ *   kind 1: check   G[r] = Op A[r] + C[r];  kres[r] = max(kres[r], ||A[r] - clip(A[r] - G[r], lb[r, k], ub[r, k])||_inf),
+ *                   k = col % nu, and +Inf for a row with a NaN or an infinite G;  G = X, which may be NULL
+ *   kind 2: store   X[r] = Op A[r]
+ * In every kind r = rows[p] for p < min(*count, max_rows) (rows NULL: r = p), and no other row is touched.  Op is n x n
+ * (n even, the INT8 pipe takes n <= 32768); A, C, X are B x n with every listed r < B; lb, ub are B x nu; kres holds B
+ * non-negative doubles as bit patterns; count is a device int.  All pointers are device memory.
+ * pipe 0 = FP64 DMMA (kind 0: the anchor GEMM of the FP64 path, kind 1: its exact check, kind 2: the plain store),
+ * pipe 1 = INT8 digit planes (kind 0: 6 levels, kinds 1 and 2: 8 levels).
+ * variant (pipe 1): -1 = the process default (NNMPC_OZ_VARIANT), 0..3 = that kernel variant.  Synchronises the stream. */
+int nnmpc_exact_apply_test(int kind, int pipe, int variant, int B, int n, int nu, const double* Op, const int* rows,
+                           const int* count, int max_rows, const double* A, const double* C, const double* lb,
+                           const double* ub, double* X, unsigned long long* kres, void* stream);
 /* nnmpc_lp_pass_probe (tools/probes/lp_pass_split.py): one tensor-core pass over B x n synthetic state with the production
  * epilogue (ms[0]), with an epilogue that only drains TMEM (ms[1]) and with the production epilogue but no TMA loads / MMAs
  * (ms[2]: the epilogue alone); then the deferred-second-term form: the one-term pass (ms[3]) and the second-term delivery

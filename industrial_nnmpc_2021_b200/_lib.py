@@ -77,6 +77,8 @@ SIGNATURES = {
     "nnmpc_lp_gemm_test": (C.c_int, [C.c_int, C.c_int, C.c_int, vp, vp, C.c_double, vp, C.c_int, vp]),
     "nnmpc_lp_pass_probe": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]),
     "nnmpc_oz_gemm_test": (C.c_int, [C.c_int, C.c_int, C.c_int, vp, vp, vp, vp]),
+    "nnmpc_exact_apply_test": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, C.c_int, vp,
+                                         vp, vp, vp, vp, vp, vp]),
     "nnmpc_gemm_tn": (C.c_int, [C.c_int, C.c_int, C.c_int, vp, C.c_longlong, vp, C.c_longlong, vp, C.c_longlong,
                                 vp, vp]),
 }

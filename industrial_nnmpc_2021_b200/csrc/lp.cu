@@ -97,11 +97,11 @@ int lp_anchor_prep(const int* rows, const int* count, int max_rows, const double
 }
 
 int lp_anchor_gemm(const int* rows, const int* count, int max_rows, const double* W, const double* Top, const double* C,
-                   LpState* s, cudaStream_t st) {
+                   double* X, int n, cudaStream_t st) {
   if (max_rows <= 0) return 0;
   GemmOperands g{};
-  g.A = W; g.lda = s->n; g.Bt = Top; g.ldb = s->n; g.M = max_rows; g.N = s->n; g.K = s->n; g.rows = rows; g.m_count = count;
-  return gemm_by_count<EpiAnchor>(g, EpiAnchor::Params{s->X.p, C, s->n}, st);
+  g.A = W; g.lda = n; g.Bt = Top; g.ldb = n; g.M = max_rows; g.N = n; g.K = n; g.rows = rows; g.m_count = count;
+  return gemm_by_count<EpiAnchor>(g, EpiAnchor::Params{X, C, n}, st);
 }
 
 int lp_dr_first(const int* rows, const int* count, int max_rows, LpState* s, double* V, double* W, const double* lb,

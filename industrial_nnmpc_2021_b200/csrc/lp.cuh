@@ -54,7 +54,7 @@ int lp_anchor_prep(const int* rows, const int* count, int max_rows, const double
                    const double* lb, const double* ub, int nu, cudaStream_t st);
 // FP64 anchor GEMM x = Top w - c over the listed rows (DMMA kernel, tile shape picked by the device-side count)
 int lp_anchor_gemm(const int* rows, const int* count, int max_rows, const double* W, const double* Top, const double* C,
-                   LpState* s, cudaStream_t st);
+                   double* X, int n, cudaStream_t st);
 // listed rows: one FP64 Douglas-Rachford step from the exact x, first fp16 increment, state := iter_state
 // pos_r: sample row -> row of the operand buffer the next pass reads (null = identity)
 int lp_dr_first(const int* rows, const int* count, int max_rows, LpState* s, double* V, double* W, const double* lb,

@@ -126,7 +126,8 @@ struct OzEpiVerify {
           const double g = v[h + k] + ql[k];
           if (p.G) p.G[base + col] = g;
           double r = fabs(z[k] - fmin(fmax(z[k] - g, l[k]), u[k]));
-          if (!(r <= 1.7e308)) r = __longlong_as_double(0x7ff0000000000000ll);   // NaN/Inf must not look converged
+          // NaN/Inf must not look converged (an infinite g clips to a bound and leaves r finite)
+          if (!(r <= 1.7e308 && fabs(g) <= 1.7e308)) r = __longlong_as_double(0x7ff0000000000000ll);
           rmax = fmax(rmax, r);
         }
       }
@@ -201,14 +202,14 @@ static oz::OzShape oz_shape(const OzOperator* op, const OzRows* r, int max_rows,
   return g;
 }
 
-// one FP64-accurate apply over the sliced rows: levels 0..LMAX through the selected kernel variant
+// one FP64-accurate apply over the sliced rows: levels 0..LMAX through kernel variant `variant` (-1: oz_variant())
 template <int LMAX, class Epi>
 static int oz_apply(const OzOperator* op, OzRows* r, int max_rows, const int* count, const typename Epi::Params& ep,
-                    int device, cudaStream_t st) {
+                    int device, cudaStream_t st, int variant = -1) {
   const int sms = device_sm_count(device);
   const oz::OzShape g = oz_shape(op, r, max_rows, count);
   cudaError_t e;
-  const int var = oz_variant();
+  const int var = variant >= 0 ? variant : oz_variant();
   if (var == 0) {
     e = oz::launch_oz_gemm<LMAX, Epi>(r->tm, op->tm, g, ep, sms, st);
     count_launch();
@@ -229,23 +230,24 @@ static int oz_apply(const OzOperator* op, OzRows* r, int max_rows, const int* co
 }
 
 int oz_anchor(const OzOperator* top, OzRows* r, const int* rows, const int* count, int max_rows, const double* W,
-              const double* C, double* X, int n, int device, cudaStream_t st) {
+              const double* C, double* X, int n, int device, cudaStream_t st, int variant) {
   if (max_rows <= 0) return 0;
   if (!top->ready || top->ncols != n || r->ncols != n || max_rows > r->cap_pad)
     return set_error(NNMPC_ERR_BADARG, "oz_anchor: operator / row planes not prepared for n = %d, %d rows", n, max_rows);
   NNMPC_TRY(oz_slice_rows(r, rows, count, max_rows, W, n, st));
-  return oz_apply<OZ_LMAX_ANCHOR, OzEpiAnchor>(top, r, max_rows, count, OzEpiAnchor::Params{X, C, rows, n}, device, st);
+  return oz_apply<OZ_LMAX_ANCHOR, OzEpiAnchor>(top, r, max_rows, count, OzEpiAnchor::Params{X, C, rows, n}, device, st,
+                                               variant);
 }
 
 int oz_verify(const OzOperator* P, OzRows* r, const int* rows, const int* count, int max_rows, const double* Z,
               const double* Ql, const double* lb, const double* ub, unsigned long long* kres, double* G, int n, int nu,
-              int device, cudaStream_t st) {
+              int device, cudaStream_t st, int variant) {
   if (max_rows <= 0) return 0;
   if (!P->ready || P->ncols != n || r->ncols != n || max_rows > r->cap_pad)
     return set_error(NNMPC_ERR_BADARG, "oz_verify: operator / row planes not prepared for n = %d, %d rows", n, max_rows);
   NNMPC_TRY(oz_slice_rows(r, rows, count, max_rows, Z, n, st));
   return oz_apply<OZ_LMAX, OzEpiVerify>(P, r, max_rows, count, OzEpiVerify::Params{Z, Ql, lb, ub, kres, G, rows, n, nu},
-                                        device, st);
+                                        device, st, variant);
 }
 
 // ---- structured-network Dense layer (mlp.cu) ---------------------------------------------------------------------
@@ -422,14 +424,14 @@ k_oz_pack_network_input(const double* __restrict__ x, const double* __restrict__
       double v1, v2;
       value(c, v1, v2);
       const double a1 = fabs(v1), a2 = fabs(v2);
-      m1 = (a1 <= m1) ? m1 : a1;       // NaN propagates
-      m2 = (a2 <= m2) ? m2 : a2;
+      m1 = oz::nan_max(m1, a1);
+      m2 = oz::nan_max(m2, a2);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const double a1 = __shfl_xor_sync(0xffffffffu, m1, o), a2 = __shfl_xor_sync(0xffffffffu, m2, o);
-      m1 = (a1 <= m1) ? m1 : a1;
-      m2 = (a2 <= m2) ? m2 : a2;
+      m1 = oz::nan_max(m1, a1);
+      m2 = oz::nan_max(m2, a2);
     }
     double inv[2], fs[2];
     const double mm[2] = {m1, m2};
@@ -495,6 +497,54 @@ int nnmpc_oz_gemm_test(int M, int N, int K, const double* A, const double* Bt, d
   cudaStreamSynchronize(st);
   op.release();
   rows.release();
+  return rc;
+}
+
+// Self test of the exact anchors and KKT checks as the closed-loop engine calls them (include/nnmpc.h).  Like the
+// engine, it slices the operator and sizes the sample planes for max_rows rows; the row list and its device-side
+// length go to the kernels unchanged.
+int nnmpc_exact_apply_test(int kind, int pipe, int variant, int B, int n, int nu, const double* Op, const int* rows,
+                           const int* count, int max_rows, const double* A, const double* C, const double* lb,
+                           const double* ub, double* X, unsigned long long* kres, void* stream) {
+  if (kind < 0 || kind > 2 || pipe < 0 || pipe > 1 || variant < -1 || variant > 3 || B <= 0 || n <= 0 || (n & 1) ||
+      max_rows <= 0 || (!rows && max_rows > B) || !Op || !A || !count || (kind != 2 && !C) || (kind != 1 && !X) ||
+      (kind == 1 && (nu <= 0 || !lb || !ub || !kres)))
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_exact_apply_test: bad argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  int dev = 0;
+  NNMPC_CUDA(cudaGetDevice(&dev));
+  int rc = 0;
+  OzOperator op;
+  OzRows r;
+  DevBuf<double> zero;
+  if (pipe == 0) {
+    GemmOperands g{};
+    g.A = A; g.lda = n; g.Bt = Op; g.ldb = n; g.M = max_rows; g.N = n; g.K = n; g.rows = rows; g.m_count = count;
+    if (kind == 0) rc = lp_anchor_gemm(rows, count, max_rows, A, Op, C, X, n, st);
+    else if (kind == 1) rc = gemm_by_count<EpiVerifyMax>(g, EpiVerifyMax::Params{A, C, lb, ub, kres, n, nu, X}, st);
+    else rc = gemm_by_count<EpiStore>(g, EpiStore::Params{X, n, nullptr, 0}, st);
+  } else {
+    rc = oz_slice_operator(Op, n, n, &op, st);
+    if (rc == 0) rc = oz_rows_ensure(&r, max_rows, n, st);
+    if (rc == 0 && kind == 0) rc = oz_anchor(&op, &r, rows, count, max_rows, A, C, X, n, dev, st, variant);
+    if (rc == 0 && kind == 1) rc = oz_verify(&op, &r, rows, count, max_rows, A, C, lb, ub, kres, X, n, nu, dev, st, variant);
+    if (rc == 0 && kind == 2) {
+      // all 8 levels through the anchor functor with c = 0: it scatters to the listed rows as the check does
+      rc = zero.ensure((size_t)B * n);
+      if (rc == 0 && cudaMemsetAsync(zero.p, 0, (size_t)B * n * sizeof(double), st) != cudaSuccess)
+        rc = set_error(NNMPC_ERR_CUDA, "nnmpc_exact_apply_test: memset failed");
+      if (rc == 0) rc = oz_slice_rows(&r, rows, count, max_rows, A, n, st);
+      if (rc == 0)
+        rc = oz_apply<OZ_LMAX, OzEpiAnchor>(&op, &r, max_rows, count, OzEpiAnchor::Params{X, zero.p, rows, n}, dev, st,
+                                            variant);
+    }
+  }
+  if (rc == 0 && cudaStreamSynchronize(st) != cudaSuccess)
+    rc = set_error(NNMPC_ERR_CUDA, "exact apply failed: %s", cudaGetErrorString(cudaGetLastError()));
+  cudaStreamSynchronize(st);
+  op.release();
+  r.release();
+  zero.release();
   return rc;
 }
 

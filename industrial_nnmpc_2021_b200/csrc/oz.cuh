@@ -52,11 +52,12 @@ int oz_pack_network_input(OzRows* r, long long B, const double* x, const double*
                           const double* xscale, int nx, int nu, int with_uprev, float* amax, cudaStream_t st);
 // x = Top w - c for the listed rows (W, C, X are B x n with the sample row as physical row)
 int oz_anchor(const OzOperator* top, OzRows* r, const int* rows, const int* count, int max_rows, const double* W,
-              const double* C, double* X, int n, int device, cudaStream_t st);
+              const double* C, double* X, int n, int device, cudaStream_t st, int variant = -1);
 // g = P z + q for the listed rows; per row ||z - clip(z - g)||_inf folded into kres (atomicMax of the bit pattern),
 // g itself into G when non-null
+// variant (both): kernel variant of the apply, -1 = the process default (NNMPC_OZ_VARIANT, read once)
 int oz_verify(const OzOperator* P, OzRows* r, const int* rows, const int* count, int max_rows, const double* Z,
               const double* Ql, const double* lb, const double* ub, unsigned long long* kres, double* G, int n, int nu,
-              int device, cudaStream_t st);
+              int device, cudaStream_t st, int variant = -1);
 
 }  // namespace nnmpc

@@ -9,8 +9,8 @@
 // scaled by a power of two into [-1/2, 1/2] and cut into signed base-128 digits
 //     a = 2^f sum_i a_i 128^-(i+1),   b = 2^e sum_j b_j 128^-(j+1),   a_i, b_j in [-64, 64]  (int8, exact)
 // so that  a . b = 2^(f+e) sum_L 128^-(L+2) sum_{i+j=L} sum_k a_i[k] b_j[k].  The inner sums are INT8 GEMMs
-// with INT32 accumulation, which is EXACT (|sum| <= 8 pairs x K x 2^12 < 2^31 for K <= 65536), so the only
-// error is the truncation at level LMAX: at most (LMAX+1) K 2^(-7 (LMAX+1) - 2) relative to 2^(f+e)
+// with INT32 accumulation, which is EXACT (|sum| <= 8 pairs x K x 2^12 <= 2^30 < 2^31 for K <= 32768, the
+// longest contraction oz_slice_operator accepts), so the only error is the truncation at level LMAX: at most (LMAX+1) K 2^(-7 (LMAX+1) - 2) relative to 2^(f+e)
 // (LMAX = 7, K = 4480: 1.2e-13 - below the rounding error of an FP64 dot product of that length), plus the
 // final FP64 summation of the levels.  36 INT8 products replace one FP64 product at 1/125 of its cost each.
 //
@@ -557,6 +557,9 @@ inline cudaError_t launch_oz_gemm2(const CUtensorMap& tmA, const CUtensorMap& tm
   return cudaGetLastError();
 }
 
+// max of |row| entries that keeps a NaN wherever it meets one ((b <= m) ? m : b alone drops an m that is NaN)
+__device__ __forceinline__ double nan_max(double m, double b) { return (b <= m || m != m) ? m : b; }
+
 // ---- slicing: one CTA per row; rows[] (optional) gathers the source rows, position p is the destination row -----
 //   src row -> 2^f (max |a| <= 2^(f-1)) and NS signed base-128 digit planes dst[(s * rows_pad + p) * ldb + k]
 template <int NS>
@@ -574,17 +577,17 @@ k_oz_slice(const int* __restrict__ rows, const int* __restrict__ count, const do
     double m = 0.0;
     for (int k = threadIdx.x; k < ncols; k += blockDim.x) {
       const double b = fabs(a[k]);
-      m = (b <= m) ? m : b;            // NaN propagates
+      m = nan_max(m, b);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const double b = __shfl_xor_sync(0xffffffffu, m, o);
-      m = (b <= m) ? m : b;
+      m = nan_max(m, b);
     }
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
     __syncthreads();
     m = red[0];
-    for (int w = 1; w < 8; ++w) m = (red[w] <= m) ? m : red[w];
+    for (int w = 1; w < 8; ++w) m = nan_max(m, red[w]);
     __syncthreads();                                        // red[] is reused by the next row
     const bool bad = !(m <= 1.7e308);                       // NaN / Inf row: the result must not look finite
     int ex = 0;
@@ -618,12 +621,12 @@ k_oz_slice_warp(const double* __restrict__ src, long long ld_src, int ncols, int
     double m = 0.0;
     for (int k = lane; k < ncols; k += 32) {
       const double b = fabs(a[k]);
-      m = (b <= m) ? m : b;            // NaN propagates
+      m = nan_max(m, b);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const double b = __shfl_xor_sync(0xffffffffu, m, o);
-      m = (b <= m) ? m : b;
+      m = nan_max(m, b);
     }
     const bool bad = !(m <= 1.7e308);
     int ex = 0;

@@ -168,6 +168,43 @@ struct EpiVerify {
   }
 };
 
+// acc = P z ; g = acc + q ; exact KKT residual ||z - clip(z - g)||_inf folded per row with atomicMax
+struct EpiVerifyMax {
+  struct Params {
+    const double* Z;
+    const double* Ql;
+    const double* lb;
+    const double* ub;
+    unsigned long long* kres;
+    int n, nu;
+    double* G;   // nullable: the exact gradient g = P z + q per element (mixed mode re-anchors x from it)
+  };
+  Params p;
+  double rmax;
+  __device__ EpiVerifyMax(const Params& p_, int, int) : p(p_), rmax(0.0) {}
+  __device__ void begin_row() { rmax = 0.0; }
+  __device__ void one(int pr, int col, double a) {
+    const long long off = (long long)pr * p.n + col;
+    const int k = col % p.nu;
+    const double z = p.Z[off], g = a + p.Ql[off];
+    if (p.G) p.G[off] = g;
+    double r = fabs(z - clipd(z - g, p.lb[(long long)pr * p.nu + k], p.ub[(long long)pr * p.nu + k]));
+    // NaN/Inf must not look converged (an infinite g clips to a bound and leaves r finite)
+    if (!(r <= 1.7e308 && fabs(g) <= 1.7e308)) r = __longlong_as_double(0x7ff0000000000000ll);
+    rmax = fmax(rmax, r);
+  }
+  __device__ void apply(int pr, int, int col, double a0, double a1, bool ok0, bool ok1) {
+    if (ok0) one(pr, col, a0);
+    if (ok1) one(pr, col + 1, a1);
+  }
+  __device__ void finish_row(int pr, int, int, bool rok) {
+    double m = rmax;
+    m = fmax(m, __shfl_xor_sync(0xffffffffu, m, 1));
+    m = fmax(m, __shfl_xor_sync(0xffffffffu, m, 2));
+    if (rok && (threadIdx.x & 3) == 0) atomicMax(p.kres + pr, (unsigned long long)__double_as_longlong(m));
+  }
+};
+
 template <class Epi>
 inline int gemm_auto(const GemmOperands& g, const typename Epi::Params& ep, cudaStream_t st) {
   cudaError_t e = use_big_tile(g.M, g.N) ? launch_gemm<TileBig, Epi>(g, ep, st)

@@ -89,42 +89,6 @@ struct nnmpc_sim {
 
 namespace nnmpc {
 
-// acc = P z ; g = acc + q ; exact KKT residual ||z - clip(z - g)||_inf folded per row with atomicMax
-struct EpiVerifyMax {
-  struct Params {
-    const double* Z;
-    const double* Ql;
-    const double* lb;
-    const double* ub;
-    unsigned long long* kres;
-    int n, nu;
-    double* G;   // nullable: the exact gradient g = P z + q per element (mixed mode re-anchors x from it)
-  };
-  Params p;
-  double rmax;
-  __device__ EpiVerifyMax(const Params& p_, int, int) : p(p_), rmax(0.0) {}
-  __device__ void begin_row() { rmax = 0.0; }
-  __device__ void one(int pr, int col, double a) {
-    const long long off = (long long)pr * p.n + col;
-    const int k = col % p.nu;
-    const double z = p.Z[off], g = a + p.Ql[off];
-    if (p.G) p.G[off] = g;
-    double r = fabs(z - clipd(z - g, p.lb[(long long)pr * p.nu + k], p.ub[(long long)pr * p.nu + k]));
-    if (!(r <= 1.7e308)) r = __longlong_as_double(0x7ff0000000000000ll);
-    rmax = fmax(rmax, r);
-  }
-  __device__ void apply(int pr, int, int col, double a0, double a1, bool ok0, bool ok1) {
-    if (ok0) one(pr, col, a0);
-    if (ok1) one(pr, col + 1, a1);
-  }
-  __device__ void finish_row(int pr, int, int, bool rok) {
-    double m = rmax;
-    m = fmax(m, __shfl_xor_sync(0xffffffffu, m, 1));
-    m = fmax(m, __shfl_xor_sync(0xffffffffu, m, 2));
-    if (rok && (threadIdx.x & 3) == 0) atomicMax(p.kres + pr, (unsigned long long)__double_as_longlong(m));
-  }
-};
-
 // ---- single-block list builders --------------------------------------------------------------
 // Ordered (ascending position) compaction by one 1024-thread block: entries with keep != 0 are
 // appended to out[] in input order; returns the new length to every thread.
@@ -927,7 +891,7 @@ static int sim_run_device(nnmpc_sim* h, int Btot, int T, double* x_io, double* u
         const bool prof64 = prof_begin(&span64, st);
         NNMPC_TRY(lp_anchor_prep(e.l_anchor, cnt, B, h->V.p, q->W0.p, &h->lps, h->lb.p, h->ub.p, nu, st));
         if (oz) NNMPC_TRY(oz_anchor(&q->ozTop, &h->ozr, e.l_anchor, cnt, B, q->W0.p, q->C.p, h->lps.X.p, n, h->device, st));
-        else NNMPC_TRY(lp_anchor_gemm(e.l_anchor, cnt, B, q->W0.p, q->Top, q->C.p, &h->lps, st));
+        else NNMPC_TRY(lp_anchor_gemm(e.l_anchor, cnt, B, q->W0.p, q->Top, q->C.p, h->lps.X.p, n, st));
         NNMPC_TRY(lp_dr_first(e.l_anchor, cnt, B, &h->lps, h->V.p, q->W0.p, h->lb.p, h->ub.p, e.state, e.it, SLOT_ITER,
                               nu, q->alpha, pos_r, st, e.need2));
         if (prof64) prof_end(span64, st, 0.0, 1, 1);

@@ -343,10 +343,12 @@ def test_generate_data_files_and_sharding_invariance(torch_cuda, cdu_small_probl
 
 
 def test_closed_loop_engine_across_tile_shapes(torch_cuda, cdu_small_problem, precision):
-    """Many trajectories of different lengths-to-convergence in one continuously batched run: the
-    batch crosses all three GEMM tile shapes (<=48, <=384, >384 rows) as trajectories finish, and
-    every trajectory must come out bitwise identical to the same trajectory run in a small batch,
-    and equal to the oracle's closed loop within the north-star tolerance."""
+    """Many trajectories of different lengths-to-convergence in one continuously batched run: as
+    trajectories finish, the row lists cross the two lower row-count windows of the FP64 GEMM tile
+    shapes (<= 48, <= 512 rows; the <= 896 and larger windows start above these 450 trajectories and
+    are reached by tests/test_gpu_exact_applies.py), and every trajectory must come out bitwise
+    identical to the same trajectory run in a small batch, and equal to the oracle's closed loop
+    within the north-star tolerance."""
     from industrial_nnmpc_2021_b200.linearMPC import OfflineSimulator
     p = cdu_small_problem
     Bn, T = 450, 5
