@@ -237,7 +237,12 @@ int nnmpc_mlp_train_step(nnmpc_mlp_t* h, long long B, const double* x, const dou
 /* current weights in Keras get_weights() layout: weights_host[l] (in_l x out_l), biases_host[l] (out_l; NULL for the last) */
 int nnmpc_mlp_get_weights(nnmpc_mlp_t* h, double* const* weights_host, double* const* biases_host);
 /* x,xs dev B x nx; uprev,us dev B x nu (uprev ignored when !with_uprev); out dev B x nu.
- * xscale dev nx or NULL (x/xscale, xs/xscale, :863-866); ulb/uub dev nu or NULL (clip, :888-892). */
+ * xscale dev nx or NULL (x/xscale, xs/xscale, :863-866); ulb/uub dev nu or NULL (clip, :888-892).
+ * Non-finite inputs: samples are independent, so a NaN or an infinity in one sample leaves every other sample
+ * bit-identical.  A sample with a NaN in x, uprev, xs or us comes back NaN in every component, in every mode and with
+ * or without the clip: ReLU and the clip keep a NaN, as the reference's np.where forms do.  An infinity gives a
+ * non-finite output wherever the float64 reference is non-finite; in modes 1 and 2 the whole sample may come back
+ * NaN, because a row holding an infinity has no finite scale. */
 int nnmpc_mlp_forward(nnmpc_mlp_t* h, long long B, const double* x, const double* uprev,
                       const double* xs, const double* us, const double* xscale, const double* ulb,
                       const double* uub, double* out, void* stream);

@@ -111,11 +111,11 @@ struct EpiStructOut {
     if ((pr & 1) || !ok0) return;
     const long long b = pr >> 1;
     double v0 = p.us[b * p.nu + col] + (a0 - b0);   // us + (out1 - out2), the reference order (:58-60)
-    if (p.ulb) v0 = fmin(fmax(v0, p.ulb[col]), p.uub[col]);
+    if (p.ulb) v0 = clip_keep_nan(v0, p.ulb[col], p.uub[col]);
     p.out[b * p.nu + col] = v0;
     if (ok1) {
       double v1 = p.us[b * p.nu + col + 1] + (a1 - b1);
-      if (p.ulb) v1 = fmin(fmax(v1, p.ulb[col + 1]), p.uub[col + 1]);
+      if (p.ulb) v1 = clip_keep_nan(v1, p.ulb[col + 1], p.uub[col + 1]);
       p.out[b * p.nu + col + 1] = v1;
     }
   }
@@ -166,7 +166,7 @@ __global__ void k_struct_out(const double* __restrict__ f, const double* __restr
     const long long b = i / nu;
     const int c = (int)(i - b * nu);
     double v = us[i] + (f[(2 * b) * nu + c] - f[(2 * b + 1) * nu + c]);
-    if (ulb) v = fmin(fmax(v, ulb[c]), uub[c]);
+    if (ulb) v = clip_keep_nan(v, ulb[c], uub[c]);
     out[i] = v;
   }
 }

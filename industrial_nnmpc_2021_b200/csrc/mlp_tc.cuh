@@ -21,15 +21,21 @@ namespace nnmpc {
 
 using MlpTile = lp::LpTile<128, lp::EPI_WARPS == 16 ? 3 : 4>;
 
-// power of two s with s * bound in [2^13, 2^14)  (fp16 max is 65504); bound = 0 or non-finite -> 1
+// power of two s with s * bound in [2^13, 2^14)  (fp16 max is 65504); bound = 0 -> 1.  A NaN or infinite bound gives a
+// NaN scale: the row it belongs to holds a NaN or an infinity, and every output of it comes back NaN through the
+// 1 / s of the epilogues, whatever the tensor cores make of the non-finite operand.
 __device__ __forceinline__ double mlp_row_scale(double bound) {
-  if (!(bound > 0.0) || !(bound <= 1.7e308)) return 1.0;
+  if (!(bound <= 1.7e308)) return __longlong_as_double(0x7ff8000000000000ll);
+  if (!(bound > 0.0)) return 1.0;
   int ex;
   frexp(bound, &ex);
   int sh = 14 - ex;
   sh = sh > 100 ? 100 : (sh < -100 ? -100 : sh);
   return ldexp(1.0, sh);
 }
+
+// fmax that keeps a NaN in either operand (fmax drops it, and the row would get a finite scale)
+__device__ __forceinline__ double max_keep_nan(double m, double b) { return (m != m || b != b) ? m + b : fmax(m, b); }
 
 __device__ __forceinline__ void mlp_split(double t, __half& hi, __half& lo) {
   hi = __double2half(t);
@@ -66,13 +72,13 @@ k_mlp_pack_tc(const double* __restrict__ x, const double* __restrict__ uprev, co
   for (int c = lane; c < o4; c += 32) {
     double v1, v2;
     value(c, v1, v2);
-    m1 = fmax(m1, fabs(v1));
-    m2 = fmax(m2, fabs(v2));
+    m1 = max_keep_nan(m1, fabs(v1));
+    m2 = max_keep_nan(m2, fabs(v2));
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
-    m1 = fmax(m1, __shfl_xor_sync(0xffffffffu, m1, o));
-    m2 = fmax(m2, __shfl_xor_sync(0xffffffffu, m2, o));
+    m1 = max_keep_nan(m1, __shfl_xor_sync(0xffffffffu, m1, o));
+    m2 = max_keep_nan(m2, __shfl_xor_sync(0xffffffffu, m2, o));
   }
   const double s1 = mlp_row_scale(m1), s2 = mlp_row_scale(m2);
   __half* r1 = A + (2 * b) * pitch;
@@ -104,7 +110,7 @@ struct EpiMlpHidden {
     const double* sc_in;   // per row: scale of the operand this pass read
     const float* amax_in;  // per row: max |entry| of that operand (unscaled)
     double* sc_out;        // per row: scale of the operand written here
-    float* amax_out;       // per row: max entry written here (atomicMax on the bit pattern; entries are >= 0)
+    float* amax_out;       // per row: max entry written here (atomicMax on the bit pattern; entries are >= 0 or +NaN)
     double inv_sw;         // 1 / weight scale
     double w1norm, bmax;   // max_j sum_i |W_ij|, max_j |b_j|
   };
@@ -133,8 +139,8 @@ struct EpiMlpHidden {
       double h = 0.0;
       if (col < N) {
         h = (double)__uint_as_float(acc[j]) * inv_in + __ldg(p.bias + col);
-        h = h > 0.0 ? h : 0.0;                                  // keras relu; NaN -> 0 is caught by the caller's checks
-        hmax = fmaxf(hmax, (float)h * 1.0000002f);
+        h = relu_keep_nan(h);                                   // keras relu; a NaN goes on to the output
+        hmax = row_max_keep_nan(hmax, (float)h * 1.0000002f);
       }
       mlp_split(h * s_out, hi[j], lo[j]);
     }
@@ -182,7 +188,7 @@ struct EpiMlpOut {
       const int col = col0 + j;
       if (ok && !(row & 1) && col < N) {
         double v = p.us[b * p.nu + col] + (f - g);              // us + (out1 - out2), the reference order (:58-60)
-        if (p.ulb) v = fmin(fmax(v, p.ulb[col]), p.uub[col]);
+        if (p.ulb) v = clip_keep_nan(v, p.ulb[col], p.uub[col]);
         p.out[b * p.nu + col] = v;
       }
     }

@@ -45,6 +45,23 @@ inline unsigned row_grid(long long max_rows) {
   return (unsigned)(max_rows < 1 ? 1 : (max_rows < cap ? max_rows : cap));
 }
 
+// Keras relu that keeps a NaN, as the reference's np.where(x < 0, 0, x) does.  Bit-identical to x > 0 ? x : 0 for
+// every other input, including -0.0 -> +0.0: the row maxima below are atomicMax on float bit patterns, where -0.0f
+// (0x80000000) would outrank every positive float.
+__device__ __forceinline__ double relu_keep_nan(double x) { return (x > 0.0 || x != x) ? x : 0.0; }
+
+// running maximum of non-negative floats that ends as the positive NaN 0x7fffffff once it meets a NaN: that bit
+// pattern outranks every other float in an atomicMax on the bits, so the row maximum of a NaN row stays NaN
+__device__ __forceinline__ float row_max_keep_nan(float m, float h) {
+  return (m != m || h != h) ? __int_as_float(0x7fffffff) : fmaxf(m, h);
+}
+
+// clip in the reference's order (np.where(u > ub, ub, u), then np.where(u < lb, lb, u)): a NaN stays NaN
+__device__ __forceinline__ double clip_keep_nan(double v, double lb, double ub) {
+  v = v > ub ? ub : v;
+  return v < lb ? lb : v;
+}
+
 // RAII-less grow-only device buffer (handles free explicitly in destroy)
 template <class T>
 struct DevBuf {

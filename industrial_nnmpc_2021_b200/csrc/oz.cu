@@ -268,7 +268,7 @@ struct OzEpiDense {
       const int col = col0 + k;
       if (col < N) {
         double h = v[k] + (p.bias ? __ldg(p.bias + col) : 0.0);
-        if (p.relu) h = h > 0.0 ? h : 0.0;
+        if (p.relu) h = relu_keep_nan(h);
         p.out[pos * p.ldo + col] = h;
       }
     }
@@ -302,7 +302,7 @@ struct OzEpiDenseF32 {
     float* H;
     long long ldh;
     const double* bias;
-    float* amax_out;       // per row: max entry written (atomicMax on the bit pattern; entries are >= 0)
+    float* amax_out;       // per row: max entry written (atomicMax on the bit pattern; entries are >= 0 or +NaN)
   };
   Params p;
   long long pos;
@@ -318,11 +318,10 @@ struct OzEpiDenseF32 {
     for (int k = 0; k < oz::CH; ++k) {
       double t = 0.0;
       if (col0 + k < N) {
-        t = v[k] + __ldg(p.bias + col0 + k);
-        t = t > 0.0 ? t : 0.0;
+        t = relu_keep_nan(v[k] + __ldg(p.bias + col0 + k));
       }
       h[k] = (float)t;
-      hmax = fmaxf(hmax, h[k]);
+      hmax = row_max_keep_nan(hmax, h[k]);    // a NaN row must reach k_oz_slice_f32 with a NaN maximum
     }
     float4* dst = reinterpret_cast<float4*>(p.H + pos * p.ldh + col0);
 #pragma unroll
@@ -348,7 +347,7 @@ k_oz_slice_f32(const float* __restrict__ H, long long ldh, int ncols, const floa
     const double inv = bad ? 0.0 : ldexp(1.0, -(ex + 1));
     for (int k = 4 * lane; k < ncols; k += 128) {          // ldh and the plane pitch are multiples of 4: whole float4 / char4
       const float4 f = *reinterpret_cast<const float4*>(a + k);
-      double t[4] = {f.x * inv, f.y * inv, f.z * inv, f.w * inv};
+      double t[4] = {bad ? 0.0 : f.x * inv, bad ? 0.0 : f.y * inv, bad ? 0.0 : f.z * inv, bad ? 0.0 : f.w * inv};
 #pragma unroll
       for (int s = 0; s < 4; ++s) {
         char4 d;

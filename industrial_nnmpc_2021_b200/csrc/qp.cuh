@@ -42,8 +42,8 @@ struct EpiStore {
       if (ok1) v1 += p.bias[col + 1];
     }
     if (p.relu) {
-      v0 = v0 > 0.0 ? v0 : 0.0;
-      v1 = v1 > 0.0 ? v1 : 0.0;
+      v0 = relu_keep_nan(v0);
+      v1 = relu_keep_nan(v1);
     }
     double* c = p.C + (long long)pr * p.ldc + col;
     if (ok1 && ((reinterpret_cast<uintptr_t>(c) & 15) == 0)) {

@@ -31,7 +31,9 @@ def _problem(rng, with_uprev, nx, nu, hidden, B):
 
 
 @pytest.mark.parametrize("with_uprev,nx,nu,hidden,B", [(True, 12, 6, [40, 32, 24], 257), (False, 12, 6, [33, 17], 64),
-                                                        (False, 252, 32, [128, 96, 64], 300)])
+                                                        (False, 252, 32, [128, 96, 64], 300),
+                                                        (False, 1, 1, [], 33),           # no hidden layer, nu = 1
+                                                        (False, 4, 3, [17], 45)])        # odd input width 11
 def test_training_steps_match_numpy_backprop_and_adam(torch_cuda, with_uprev, nx, nu, hidden, B):
     from industrial_nnmpc_2021_b200.LinearMPCLayers import RegulatorLayerWithUprev, RegulatorLayerWithoutUprev
     rng = np.random.default_rng(nx + nu + B)
