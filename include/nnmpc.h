@@ -98,7 +98,8 @@ int nnmpc_qp_solve(nnmpc_qp_t* h, int B, const double* x0, const double* lb, con
 int nnmpc_qp_solve_host(nnmpc_qp_t* h, int B, const double* x0, const double* lb, const double* ub,
                         double* u, double* cost, double* kkt, int* iters, double tol, int max_iter);
 
-/* ---- target selector:  TargetSelector.solve (lib/linearMPC.py:298-311), H empty, A stable ------
+/* ---- target selector:  TargetSelector.solve (lib/linearMPC.py:298-311) -------------------------
+ * nnmpc_ts_create: H empty and I - A invertible.
  * Reduced exactly to the nu-dim box QP  min 1/2 us'Ht us + (Fy ysp + Fd d + f0)'us,
  * xs = Gx us + Gd d  (Gx = (I-A)^-1 B, Gd = (I-A)^-1 Bd).  nu <= 32. */
 int nnmpc_ts_create(nnmpc_ts_t** out, int nx, int nu, int ny, int nd, const double* Ht_host,
@@ -115,6 +116,26 @@ int nnmpc_ts_create(nnmpc_ts_t** out, int nx, int nu, int ny, int nd, const doub
 int nnmpc_ts_set_output_bounds(nnmpc_ts_t* h, const double* Hinv_host, const double* Abar_host, const double* AH_host,
                                const double* Mbar_host, const double* Ryd_host, const double* ylb_host,
                                const double* yub_host);
+/* Targets with pinned outputs (H non-empty: H C xs = H (ysp - Cd dhat)) or an integrating plant (I - A singular),
+ * where xs cannot be eliminated through (I - A)^-1.  With s = [ysp; dhat] (ny + nd) and an orthonormal basis Z of
+ * null(tA), tA = [I-A, -B; HC, 0] of full row rank, the targets are [xs; us] = K s + Z v, K = tA^+ tb, for the nw =
+ * nu - nz remaining variables v, which solve
+ *     min 1/2 v'(Z'PZ) v + (Fy ysp + Fd dhat + f0)'v   s.t.  lo0 - R s <= Abar v <= hi0 - R s   (mb rows).
+ * Host arrays, row-major:  Hinv = (Z'PZ)^-1 (nw x nw), Abar (mb x nw), AH = Abar Hinv (mb x nw), Mbar = Abar Hinv Abar'
+ * (mb x mb), Fy (nw x ny), Fd (nw x nd), f0 (nw), R (mb x (ny + nd)), lo0, hi0 (mb), Kx (nx x (ny + nd)),
+ * Ku (nu x (ny + nd)), Zx (nx x nw), Zu (nu x nw), ulb, uub (nu).  The last nu rows are the input box in input order
+ * (Abar = Zu, R = Ku, lo0 = ulb, hi0 = uub); the first mb - nu rows are free to use, e.g. output bounds
+ * (Abar = C Zx, R = C Kx + [0 Cd], lo0 = ylb, hi0 = yub).  nu <= 32, 0 <= nw <= nu, nu <= mb <= 160.
+ * nw = 0 is valid: the target is K s, and a sample whose K s violates a row is infeasible; the arrays of size zero
+ * (Hinv, Abar, AH, Fy, Fd, f0, Zx, Zu) may then be NULL.  Solved by the dual active-set method of
+ * nnmpc_ts_set_output_bounds; nnmpc_ts_solve*, nnmpc_sim_* and nnmpc_online_* take the handle unchanged, and an
+ * infeasible sample raises NNMPC_WARN_TARGET and carries a negative iteration count. */
+int nnmpc_ts_create_reduced(nnmpc_ts_t** out, int nx, int nu, int ny, int nd, int nw, int mb, const double* Hinv_host,
+                            const double* Abar_host, const double* AH_host, const double* Mbar_host,
+                            const double* Fy_host, const double* Fd_host, const double* f0_host, const double* R_host,
+                            const double* lo0_host, const double* hi0_host, const double* Kx_host,
+                            const double* Ku_host, const double* Zx_host, const double* Zu_host,
+                            const double* ulb_host, const double* uub_host, int device);
 int nnmpc_ts_destroy(nnmpc_ts_t* h);
 /* ysp: dev B rows of ny doubles, row stride ysp_stride (doubles); d likewise. */
 /* iters (nullable): active-set steps per sample; a sample whose solve stalled at the step cap or went

@@ -39,6 +39,8 @@ SIGNATURES = {
     "nnmpc_ts_create": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp, vp,
                                   vp, C.c_int]),
     "nnmpc_ts_set_output_bounds": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, vp]),
+    "nnmpc_ts_create_reduced": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+                                + [vp] * 16 + [C.c_int]),
     "nnmpc_ts_destroy": (C.c_int, [vp]),
     "nnmpc_ts_solve": (C.c_int, [vp, C.c_int, vp, C.c_longlong, vp, C.c_longlong, vp, vp, vp, vp]),
     "nnmpc_ts_solve_host": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, vp]),

@@ -3,7 +3,7 @@
 // Replaces TargetSelector.solve (/root/reference/lib/linearMPC.py:298-311), which calls cvxopt on
 //     min_(xs,us) 1/2|us-usp|^2_Rs + 1/2|C xs + Cd d - ysp|^2_Qs
 //     s.t. (I-A) xs - B us = Bd d ,  ulb <= us <= uub                 (:182-187, H empty)
-// With A open-loop stable the equality eliminates xs = Gx us + Gd d and leaves an nu-dimensional
+// With I - A invertible the equality eliminates xs = Gx us + Gd d and leaves an nu-dimensional
 // strictly convex box QP,  min 1/2 us'Ht us + f'us,  f = Fy ysp + Fd d + f0  (operators built on
 // the host, see linearMPC.TargetSelector).  nu <= 32, so lane i of a warp owns variable i and the
 // QP is solved EXACTLY by a primal active-set method: equality-constrained solves through a
@@ -31,10 +31,12 @@ struct TsParams {
   int indexed;
   TsIndex ix;
   int* fail;   // nullable device flag, set when a solve stalls at the iteration cap or produces non-finite targets
-  int given;   // 1: us (and iters) were written by k_ts_general; this kernel only forms xs and the fused outputs
-  // output-constrained targets (k_ts_general)
-  int mb;
-  const double *Hinv, *Abar, *AH, *Mbar, *Ryd, *ylb, *yub;
+  // 1: us (and iters) were written by k_ts_general; this kernel only forms xs and the fused outputs
+  // 2: xs was written too (reduced targets); this kernel only forms the fused outputs
+  int given;
+  // k_ts_general (see nnmpc_ts in ts.cuh)
+  int nw, mb, nR, rld, rny, reduced;
+  const double *Hinv, *Abar, *AH, *Mbar, *R, *lo0, *hi0, *Kx, *Ku, *Zx, *Zu;
 };
 
 __device__ __forceinline__ double warp_min_d(double v) {
@@ -54,7 +56,8 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_target_selector(TsParams p) {
   __shared__ double uw[TS_WARPS][32];
   const int nu = p.nu, nx = p.nx, ny = p.ny, nd = p.nd;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int i = threadIdx.x; i < nu * nu; i += blockDim.x) Hs[(i / nu) * TS_LD + (i % nu)] = p.Ht[i];
+  if (!p.given)
+    for (int i = threadIdx.x; i < nu * nu; i += blockDim.x) Hs[(i / nu) * TS_LD + (i % nu)] = p.Ht[i];
   __syncthreads();
   double* S = Sw[warp];
   double* uvec = uw[warp];
@@ -83,7 +86,7 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_target_selector(TsParams p) {
       same = __all_sync(FULLMASK, eq);
     }
     double f = 0.0;
-    if (act && !same) {
+    if (act && !same && !p.given) {      // (with given targets Fy / Fd / f0 may be k_ts_general's nw-row operators)
       f = p.f0[lane];
       const double* fy = p.Fy + (long long)lane * ny;
       for (int y = 0; y < ny; ++y) f += fy[y] * ysp[y];
@@ -206,11 +209,15 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_target_selector(TsParams p) {
     const TsFused& F = p.f;
     for (int r = lane; r < nx; r += 32) {
       double acc = 0.0;
-      const double* gx = p.Gx + (long long)r * nu;
-      for (int j = 0; j < nu; ++j) acc += gx[j] * uvec[j];
-      const double* gd = p.Gd + (long long)r * nd;
-      for (int k = 0; k < nd; ++k) acc += gd[k] * dd[k];
-      p.xs[(long long)b * p.xs_stride + r] = acc;
+      if (p.given == 2) {
+        acc = p.xs[(long long)b * p.xs_stride + r];
+      } else {
+        const double* gx = p.Gx + (long long)r * nu;
+        for (int j = 0; j < nu; ++j) acc += gx[j] * uvec[j];
+        const double* gd = p.Gd + (long long)r * nd;
+        for (int k = 0; k < nd; ++k) acc += gd[k] * dd[k];
+        p.xs[(long long)b * p.xs_stride + r] = acc;
+      }
       if (p.fused) {
         const double xv = F.x[s * nx + r];
         F.x0[s * F.nxa_ld + r] = xv - acc;
@@ -244,7 +251,15 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_target_selector(TsParams p) {
 // one |W| x |W| Cholesky in shared memory (|W| <= nu <= 32) and a few gathers.  The final point is re-solved from its
 // working set, so rounding does not accumulate over the steps.  An infeasible sample (no step length exists) or one
 // that runs out of steps raises the fail flag and carries a negative iteration count - cvxopt would report a status.
-constexpr int TS_MAXC = 160;      // ny + nu
+//
+// ---- reduced targets: H non-empty (H C xs = H (ysp - Cd d), linearMPC.py:254-267) or I - A singular ----
+// xs cannot be eliminated through (I - A)^-1 there.  The host takes an orthonormal basis Z of null(tA) instead and
+// writes [xs; us] = K s + Z v, s = [ysp; d], K = tA^+ tb, so the equalities hold for every v of the nw = nu - nz
+// remaining dimensions.  The same kernel then solves over v: lane i owns v_i (i < nw), the mb = nu (+ ny) rows are
+// [C Zx; Zu] with the per-sample offsets R s, R = [C Kx + [0 Cd]; Ku], and the warp reconstructs xs and us from the
+// final v.  The output-bounded mode above is the case Z = [Gx; I], v = us.  nw = 0 leaves no freedom: the target is
+// K s, returned when it satisfies the rows and flagged infeasible otherwise.
+constexpr int TS_MAXC = 160;      // mb
 
 __device__ __forceinline__ double warp_sum_d(double v) {
 #pragma unroll
@@ -290,7 +305,9 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
   __shared__ double uw[TS_WARPS][32], fw[TS_WARPS][32], lamw[TS_WARPS][32], rw[TS_WARPS][32];
   __shared__ double blo[TS_WARPS][TS_MAXC], bhi[TS_WARPS][TS_MAXC];
   __shared__ int widx[TS_WARPS][32], wsgn[TS_WARPS][32];
-  const int nu = p.nu, ny = p.ny, nd = p.nd, mb = p.mb;
+  const int nu = p.nu, nx = p.nx, ny = p.ny, nd = p.nd, mb = p.mb, nw = p.nw;
+  const int row_u = mb - nu;      // first input row
+  const int ns = ny + nd;         // columns of Kx / Ku
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   double* S = Sw[warp];
   double* uvec = uw[warp];
@@ -301,8 +318,8 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
   double* hi = bhi[warp];
   int* wi = widx[warp];
   int* ws = wsgn[warp];
-  const bool act = lane < nu;
-  const int maxit = 8 * (nu + 8) + 2 * ny;
+  const bool act = lane < nw;
+  const int maxit = 8 * (nu + 8) + 2 * row_u;
   const double INF = __longlong_as_double(0x7ff0000000000000ll);
 
   const int Bn = p.indexed && p.ix.count ? min(*p.ix.count, p.B) : p.B;
@@ -322,21 +339,23 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
     }
     fvec[lane] = f;
     for (int i = lane; i < mb; i += 32) {
-      if (i < ny) {
+      if (i < p.nR) {
         double r = 0.0;
-        for (int k = 0; k < nd; ++k) r += p.Ryd[(long long)i * nd + k] * dd[k];
-        lo[i] = p.ylb[i] - r;
-        hi[i] = p.yub[i] - r;
+        const double* Ri = p.R + (long long)i * p.rld;
+        for (int y = 0; y < p.rny; ++y) r += Ri[y] * ysp[y];
+        for (int k = 0; k < nd; ++k) r += Ri[p.rny + k] * dd[k];
+        lo[i] = p.lo0[i] - r;
+        hi[i] = p.hi0[i] - r;
       } else {
-        lo[i] = p.ulb[i - ny];
-        hi[i] = p.uub[i - ny];
+        lo[i] = p.lo0[i];
+        hi[i] = p.hi0[i];
       }
     }
     __syncwarp();
     // unconstrained minimiser
     double u = 0.0;
     if (act)
-      for (int j = 0; j < nu; ++j) u -= p.Hinv[(long long)lane * nu + j] * fvec[j];
+      for (int j = 0; j < nw; ++j) u -= p.Hinv[(long long)lane * nw + j] * fvec[j];
     int nW = 0, it = 0;
     bool done = false, failed = false;
     for (; it < maxit && !done && !failed; ++it) {
@@ -347,8 +366,8 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
       int bi = -1, bs = 0;
       for (int i = lane; i < mb; i += 32) {
         double val = 0.0, mag = 0.0;
-        const double* a = p.Abar + (long long)i * nu;
-        for (int k = 0; k < nu; ++k) {
+        const double* a = p.Abar + (long long)i * nw;
+        for (int k = 0; k < nw; ++k) {
           const double t = a[k] * uvec[k];
           val += t;
           mag += fabs(t);
@@ -369,7 +388,7 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
       double vp = vmax;
       double lam_p = 0.0;
       const double mpp = p.Mbar[(long long)ip * mb + ip];
-      for (int inner = 0; inner <= 2 * nu + 2; ++inner) {
+      for (int inner = 0; inner <= 2 * nw + 2; ++inner) {
         // d = A_W Hinv a_p, S = A_W Hinv A_W'
         double dj = 0.0;
         if (lane < nW) {
@@ -384,8 +403,8 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
         // z = Hinv a_p - Hinv A_W' r  (lane k holds z_k),  a_p'z = Mbar[p][p] - d'r
         double z = 0.0;
         if (act) {
-          z = (double)sp * p.AH[(long long)ip * nu + lane];
-          for (int j = 0; j < nW; ++j) z -= rvec[j] * (double)ws[j] * p.AH[(long long)wi[j] * nu + lane];
+          z = (double)sp * p.AH[(long long)ip * nw + lane];
+          for (int j = 0; j < nW; ++j) z -= rvec[j] * (double)ws[j] * p.AH[(long long)wi[j] * nw + lane];
         }
         const double apz = mpp - warp_sum_d(lane < nW ? dj * rj : 0.0);
         // step lengths
@@ -417,7 +436,7 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
         if (lane >= jb && lane + 1 < nW) { wi[lane] = wi_n; ws[lane] = ws_n; lam[lane] = lam_n; }
         --nW;
         __syncwarp();
-        if (inner == 2 * nu + 2) failed = true;
+        if (inner == 2 * nw + 2) failed = true;
       }
     }
     if (!done && !failed) failed = true;      // out of steps
@@ -427,7 +446,7 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
       if (lane < nW) {
         const long long ij = wi[lane];
         double ahf = 0.0;
-        for (int k = 0; k < nu; ++k) ahf += p.AH[ij * nu + k] * fvec[k];
+        for (int k = 0; k < nw; ++k) ahf += p.AH[ij * nw + k] * fvec[k];
         const double bw = ws[lane] > 0 ? hi[ij] : -lo[ij];
         rhs = -(bw + (double)ws[lane] * ahf);
         for (int k = 0; k <= lane; ++k) S[lane * TS_LD + k] = (double)(ws[lane] * ws[k]) * p.Mbar[ij * mb + wi[k]];
@@ -438,23 +457,50 @@ __global__ void __launch_bounds__(TS_WARPS * 32) k_ts_general(TsParams p) {
       __syncwarp();
       if (act) {
         double un = 0.0;
-        for (int j = 0; j < nu; ++j) un -= p.Hinv[(long long)lane * nu + j] * fvec[j];
-        for (int j = 0; j < nW; ++j) un -= rvec[j] * (double)ws[j] * p.AH[(long long)wi[j] * nu + lane];
+        for (int j = 0; j < nw; ++j) un -= p.Hinv[(long long)lane * nw + j] * fvec[j];
+        for (int j = 0; j < nW; ++j) un -= rvec[j] * (double)ws[j] * p.AH[(long long)wi[j] * nw + lane];
         u = un;
       }
-      // inputs whose own bound is in the working set sit on it exactly; the others are inside the box up to the
-      // violation tolerance (1e-11 relative) and are clipped to it, so that the regulator's shifted bounds
-      // ulb - us <= 0 <= uub - us keep their signs
-      uvec[lane] = u;
+    }
+    uvec[lane] = u;
+    __syncwarp();
+    bool xs_bad = false;
+    if (p.reduced) {      // xs = Kx s + Zx v, us = Ku s + Zu v
+      for (int r = lane; r < nx; r += 32) {
+        double acc = 0.0;
+        const double* kx = p.Kx + (long long)r * ns;
+        for (int y = 0; y < ny; ++y) acc += kx[y] * ysp[y];
+        for (int k = 0; k < nd; ++k) acc += kx[ny + k] * dd[k];
+        const double* zx = p.Zx + (long long)r * nw;
+        for (int j = 0; j < nw; ++j) acc += zx[j] * uvec[j];
+        p.xs[(long long)b * p.xs_stride + r] = acc;
+        xs_bad = xs_bad || !(fabs(acc) <= 1.7e308);
+      }
+      double un = 0.0;
+      if (lane < nu) {
+        const double* ku = p.Ku + (long long)lane * ns;
+        for (int y = 0; y < ny; ++y) un += ku[y] * ysp[y];
+        for (int k = 0; k < nd; ++k) un += ku[ny + k] * dd[k];
+        const double* zu = p.Zu + (long long)lane * nw;
+        for (int j = 0; j < nw; ++j) un += zu[j] * uvec[j];
+      }
       __syncwarp();
-      if (lane < nW && wi[lane] >= ny) uvec[wi[lane] - ny] = ws[lane] > 0 ? hi[wi[lane]] : lo[wi[lane]];
+      uvec[lane] = u = un;
+      __syncwarp();
+    }
+    // inputs whose own bound is in the working set sit on it exactly; the others are inside the box up to the
+    // violation tolerance (1e-11 relative) and are clipped to it, so that the regulator's shifted bounds
+    // ulb - us <= 0 <= uub - us keep their signs
+    if (done && nW > 0) {
+      if (lane < nW && wi[lane] >= row_u) uvec[wi[lane] - row_u] = ws[lane] > 0 ? p.uub[wi[lane] - row_u] : p.ulb[wi[lane] - row_u];
       __syncwarp();
       u = uvec[lane];
     }
-    if (act && done) u = fmin(fmax(u, p.ulb[lane]), p.uub[lane]);
-    const bool bad = failed || __any_sync(FULLMASK, act && !(fabs(u) <= 1.7e308));
+    const bool inp = lane < nu;
+    if (inp && done) u = fmin(fmax(u, p.ulb[lane]), p.uub[lane]);
+    const bool bad = failed || __any_sync(FULLMASK, xs_bad || (inp && !(fabs(u) <= 1.7e308)));
     if (bad && p.fail && lane == 0) atomicExch(p.fail, 1);
-    if (act) p.us[(long long)b * p.us_stride + lane] = u;
+    if (inp) p.us[(long long)b * p.us_stride + lane] = u;
     if (p.iters && lane == 0) p.iters[(long long)b * p.iters_stride] = bad ? -it - 1 : it;
     __syncwarp();
   }
@@ -478,12 +524,15 @@ int ts_solve_device(nnmpc_ts* h, int B, const double* ysp, long long ysp_stride,
   p.fail = fail_flag;
   int blocks = (B + TS_WARPS - 1) / TS_WARPS;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  if (h->general) {      // output-constrained targets: the dual active-set kernel solves, the kernel below forms xs / fused outputs
-    p.mb = h->mb; p.Hinv = h->Hinv; p.Abar = h->Abar; p.AH = h->AH; p.Mbar = h->Mbar; p.Ryd = h->Ryd; p.ylb = h->ylb; p.yub = h->yub;
+  if (h->general) {      // the dual active-set kernel solves; the kernel below forms xs (unless reduced) and the fused outputs
+    p.nw = h->nw; p.mb = h->mb; p.nR = h->nR; p.rld = h->rld; p.rny = h->rny; p.reduced = h->reduced ? 1 : 0;
+    p.Hinv = h->Hinv; p.Abar = h->Abar; p.AH = h->AH; p.Mbar = h->Mbar; p.R = h->R; p.lo0 = h->lo0; p.hi0 = h->hi0;
+    p.Kx = h->Kx; p.Ku = h->Ku; p.Zx = h->Zx; p.Zu = h->Zu;
     k_ts_general<<<blocks, TS_WARPS * 32, 0, st>>>(p);
     count_launch();
     NNMPC_CUDA(cudaGetLastError());
-    p.given = 1;
+    p.given = h->reduced ? 2 : 1;
+    if (h->reduced && !fused) return 0;      // xs and us are final
   }
   k_target_selector<<<blocks, TS_WARPS * 32, 0, st>>>(p);
   count_launch();
@@ -511,8 +560,7 @@ int nnmpc_ts_create(nnmpc_ts_t** out, int nx, int nu, int ny, int nd, const doub
   DeviceGuard dg(device);
   nnmpc_ts* h = new (std::nothrow) nnmpc_ts();
   if (!h) return set_error(NNMPC_ERR_NOMEM, "out of host memory");
-  h->nx = nx; h->nu = nu; h->ny = ny; h->nd = nd; h->device = device;
-  h->Ht = h->Fy = h->Fd = h->f0 = h->Gx = h->Gd = h->ulb = h->uub = nullptr;
+  h->nx = nx; h->nu = nu; h->ny = ny; h->nd = nd; h->nw = nu; h->device = device;
   int rc = upload(&h->Ht, Ht, (size_t)nu * nu);
   if (rc == 0) rc = upload(&h->Fy, Fy, (size_t)nu * ny);
   if (rc == 0) rc = upload(&h->Fd, Fd, (size_t)nu * (nd > 0 ? nd : 1));
@@ -536,7 +584,8 @@ int nnmpc_ts_destroy(nnmpc_ts_t* h) {
   DeviceGuard dg(h->device);
   cudaFree(h->Ht); cudaFree(h->Fy); cudaFree(h->Fd); cudaFree(h->f0); cudaFree(h->Gx); cudaFree(h->Gd);
   cudaFree(h->ulb); cudaFree(h->uub);
-  cudaFree(h->Hinv); cudaFree(h->Abar); cudaFree(h->AH); cudaFree(h->Mbar); cudaFree(h->Ryd); cudaFree(h->ylb); cudaFree(h->yub);
+  cudaFree(h->Hinv); cudaFree(h->Abar); cudaFree(h->AH); cudaFree(h->Mbar); cudaFree(h->R); cudaFree(h->lo0); cudaFree(h->hi0);
+  cudaFree(h->Kx); cudaFree(h->Ku); cudaFree(h->Zx); cudaFree(h->Zu);
   if (h->fail) cudaFree(h->fail);
   h->hysp.release(); h->hd.release(); h->hxs.release(); h->hus.release(); h->hiters.release();
   delete h;
@@ -556,11 +605,71 @@ int nnmpc_ts_set_output_bounds(nnmpc_ts_t* h, const double* Hinv, const double* 
   NNMPC_TRY(upload(&h->Abar, Abar, (size_t)mb * nu));
   NNMPC_TRY(upload(&h->AH, AH, (size_t)mb * nu));
   NNMPC_TRY(upload(&h->Mbar, Mbar, (size_t)mb * mb));
-  NNMPC_TRY(upload(&h->Ryd, Ryd, ny * nd));
-  NNMPC_TRY(upload(&h->ylb, ylb, ny));
-  NNMPC_TRY(upload(&h->yub, yub, ny));
-  h->mb = mb;
+  NNMPC_TRY(upload(&h->R, Ryd, ny * nd));
+  // row bounds [ylb; ulb], [yub; uub]; only the ny output rows carry an offset, Ryd d
+  NNMPC_CUDA(cudaMalloc((void**)&h->lo0, (size_t)mb * 8));
+  NNMPC_CUDA(cudaMalloc((void**)&h->hi0, (size_t)mb * 8));
+  NNMPC_CUDA(cudaMemcpy(h->lo0, ylb, ny * 8, cudaMemcpyHostToDevice));
+  NNMPC_CUDA(cudaMemcpy(h->hi0, yub, ny * 8, cudaMemcpyHostToDevice));
+  NNMPC_CUDA(cudaMemcpy(h->lo0 + ny, h->ulb, nu * 8, cudaMemcpyDeviceToDevice));
+  NNMPC_CUDA(cudaMemcpy(h->hi0 + ny, h->uub, nu * 8, cudaMemcpyDeviceToDevice));
+  h->mb = mb; h->nR = h->ny; h->rld = h->nd; h->rny = 0;
   h->general = true;
+  return 0;
+}
+
+// Uploads n doubles; an empty array (nw = 0) stays a null device pointer and may be null on the host.
+static int upload_opt(double** dst, const double* host, size_t n) {
+  if (n == 0) return 0;
+  return upload(dst, host, n);
+}
+
+int nnmpc_ts_create_reduced(nnmpc_ts_t** out, int nx, int nu, int ny, int nd, int nw, int mb, const double* Hinv,
+                            const double* Abar, const double* AH, const double* Mbar, const double* Fy, const double* Fd,
+                            const double* f0, const double* R, const double* lo0, const double* hi0, const double* Kx,
+                            const double* Ku, const double* Zx, const double* Zu, const double* ulb, const double* uub,
+                            int device) {
+  if (nu < 1 || nu > 32) return set_error(NNMPC_ERR_UNSUPPORTED, "nnmpc_ts_create_reduced: nu=%d not in [1,32]", nu);
+  if (nx < 1 || ny < 1 || nd < 0 || nw < 0 || nw > nu || mb < nu)
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_ts_create_reduced: bad sizes");
+  if (mb > TS_MAXC) return set_error(NNMPC_ERR_UNSUPPORTED, "nnmpc_ts_create_reduced: mb = %d exceeds %d", mb, TS_MAXC);
+  if (!out || !Mbar || !R || !lo0 || !hi0 || !Kx || !Ku || !ulb || !uub ||
+      (nw > 0 && (!Hinv || !Abar || !AH || !Fy || !f0 || !Zx || !Zu || (nd > 0 && !Fd))))
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_ts_create_reduced: null argument");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return set_error(NNMPC_ERR_CUDA, "nnmpc_ts_create_reduced: no CUDA device (this library has no CPU fallback)");
+  if (device < 0 || device >= ndev) return set_error(NNMPC_ERR_BADARG, "nnmpc_ts_create_reduced: bad device %d", device);
+  DeviceGuard dg(device);
+  nnmpc_ts* h = new (std::nothrow) nnmpc_ts();
+  if (!h) return set_error(NNMPC_ERR_NOMEM, "out of host memory");
+  h->nx = nx; h->nu = nu; h->ny = ny; h->nd = nd; h->nw = nw; h->device = device;
+  const size_t w = (size_t)nw, m = (size_t)mb, ns = (size_t)(ny + nd);
+  int rc = upload_opt(&h->Hinv, Hinv, w * w);
+  if (rc == 0) rc = upload_opt(&h->Abar, Abar, m * w);
+  if (rc == 0) rc = upload_opt(&h->AH, AH, m * w);
+  if (rc == 0) rc = upload(&h->Mbar, Mbar, m * m);
+  if (rc == 0) rc = upload_opt(&h->Fy, Fy, w * ny);
+  if (rc == 0) rc = upload_opt(&h->Fd, Fd, w * nd);
+  if (rc == 0) rc = upload_opt(&h->f0, f0, w);
+  if (rc == 0) rc = upload(&h->R, R, m * ns);
+  if (rc == 0) rc = upload(&h->lo0, lo0, m);
+  if (rc == 0) rc = upload(&h->hi0, hi0, m);
+  if (rc == 0) rc = upload(&h->Kx, Kx, (size_t)nx * ns);
+  if (rc == 0) rc = upload(&h->Ku, Ku, (size_t)nu * ns);
+  if (rc == 0) rc = upload_opt(&h->Zx, Zx, (size_t)nx * w);
+  if (rc == 0) rc = upload_opt(&h->Zu, Zu, (size_t)nu * w);
+  if (rc == 0) rc = upload(&h->ulb, ulb, (size_t)nu);
+  if (rc == 0) rc = upload(&h->uub, uub, (size_t)nu);
+  if (rc == 0 && cudaMalloc((void**)&h->fail, sizeof(int)) != cudaSuccess)
+    rc = set_error(NNMPC_ERR_NOMEM, "nnmpc_ts_create_reduced: cudaMalloc failed: %s", cudaGetErrorString(cudaGetLastError()));
+  if (rc < 0) {
+    nnmpc_ts_destroy(h);
+    return rc;
+  }
+  h->mb = mb; h->nR = mb; h->rld = ny + nd; h->rny = ny;
+  h->general = h->reduced = true;
+  *out = h;
   return 0;
 }
 

@@ -4,13 +4,20 @@
 
 struct nnmpc_ts {
   int nx, nu, ny, nd, device;
+  int nw = 0;                                        // variables of the QP k_ts_general solves (nu unless reduced)
   int* fail = nullptr;                               // device flag: some solve of the last call missed its optimum
-  double *Ht, *Fy, *Fd, *f0, *Gx, *Gd, *ulb, *uub;  // device operators
-  // output-constrained targets (nnmpc_ts_set_output_bounds): constraint rows Abar = [C Gx; I] (mb x nu), Hinv = Ht^-1,
-  // AH = Abar Hinv, Mbar = Abar Hinv Abar', Ryd = C Gd + Cd (ny x nd), output bounds ylb, yub (ny)
-  bool general = false;
-  int mb = 0;
-  double *Hinv = nullptr, *Abar = nullptr, *AH = nullptr, *Mbar = nullptr, *Ryd = nullptr, *ylb = nullptr, *yub = nullptr;
+  double *Ht = nullptr, *Fy = nullptr, *Fd = nullptr, *f0 = nullptr, *Gx = nullptr, *Gd = nullptr;   // device operators
+  double *ulb = nullptr, *uub = nullptr;
+  // k_ts_general (output-constrained or reduced targets): min 1/2 v'Hinv^-1 v + (Fy ysp + Fd d + f0)'v over nw variables
+  // s.t. lo0_i - R_i s <= Abar_i v <= hi0_i - R_i s (mb rows, the last nu of them the inputs'), AH = Abar Hinv,
+  // Mbar = Abar Hinv Abar'.  Rows i < nR carry the offset R_i s: row i of R (row stride rld) holds rny coefficients on
+  // ysp (0 or ny) followed by nd on d.
+  //   output bounds (nnmpc_ts_set_output_bounds): v = us, Abar = [C Gx; I], R = C Gd + Cd on the ny output rows only
+  //   reduced (nnmpc_ts_create_reduced): [xs; us] = K s + Z v with s = [ysp; d]; the kernel also forms xs and us
+  bool general = false, reduced = false;
+  int mb = 0, nR = 0, rld = 0, rny = 0;
+  double *Hinv = nullptr, *Abar = nullptr, *AH = nullptr, *Mbar = nullptr, *R = nullptr, *lo0 = nullptr, *hi0 = nullptr;
+  double *Kx = nullptr, *Ku = nullptr, *Zx = nullptr, *Zu = nullptr;
   nnmpc::DevBuf<double> hysp, hd, hxs, hus;          // staging for the host entry point
   nnmpc::DevBuf<int> hiters;
 };

@@ -105,12 +105,17 @@ class TargetSelector:
         min_(xs,us) |us-usp|^2_Rs + |C xs + Cd dhat - ysp|^2_Qs
         s.t. [I-A, -B; HC, 0][xs; us] = [Bd dhat; H(ysp - Cd dhat)],  ulb <= us <= uub
 
-    Supported configuration: ``H`` empty (both reference examples: cstrs_parameters.py:278,
-    cdu_parameters.py:78), ``I - A`` invertible (any A without an eigenvalue at 1, stable or not), ``Nu <= 32``.
-    Then ``xs = Gx us + Gd dhat`` and the problem is an exactly equivalent ``Nu``-dimensional QP (see csrc/ts.cu): a
-    box QP solved by a primal active-set method, or - with output bounds ``ylb <= C xs + Cd dhat <= yub``
-    (linearMPC.py:242-248, :284-288; ``Ny + Nu <= 160``) - a QP over ``Ny + Nu`` two-sided rows solved by a dual
-    active-set method.  An infeasible or stalled solve raises ``NnmpcError`` (cvxopt would report a status).
+    ``Nu <= 32``.  With ``H`` empty (both reference examples: cstrs_parameters.py:278, cdu_parameters.py:78) and
+    ``I - A`` invertible (any A without an eigenvalue at 1, stable or not), ``xs = Gx us + Gd dhat`` and the problem is
+    an exactly equivalent ``Nu``-dimensional QP (see csrc/ts.cu): a box QP solved by a primal active-set method, or -
+    with output bounds ``ylb <= C xs + Cd dhat <= yub`` (linearMPC.py:242-248, :284-288; ``Ny + Nu <= 160``) - a QP
+    over ``Ny + Nu`` two-sided rows solved by a dual active-set method.
+    With ``H`` non-empty (chosen outputs reach their set-points exactly) or an integrating plant (``I - A`` singular)
+    the equalities are eliminated through a null-space basis instead, ``[xs; us] = K s + Z v`` with ``s = [ysp; dhat]``
+    (``reduced`` is True, operators from ``_setup_reduction``), and the same dual active-set method solves over the
+    ``Nu - Nz`` entries of ``v``.  ``tA`` must then have full row rank and the reduced Hessian ``Z'PZ`` must be positive
+    definite (a unique target); the constructor refuses other problems.
+    An infeasible or stalled solve raises ``NnmpcError`` (cvxopt would report a status).
     """
 
     def __init__(self, *, A, B, C, H, Bd, Cd, usp, Rs, Qs, ulb, uub, ylb=None, yub=None, device=None):
@@ -120,14 +125,8 @@ class TargetSelector:
         self.usp = usp
         self.ysp, self.dhats, self.xs, self.us = [], [], [], []
         self.ulb, self.uub, self.ylb, self.yub = ulb, uub, ylb, yub
-        if self.Nz != 0:
-            raise NotImplementedError("TargetSelector on the GPU supports H empty only "
-                                      "(the configuration of both reference examples)")
         if (ylb is None) != (yub is None):
             ylb = yub = self.ylb = self.yub = None      # the reference uses output bounds only when both are given (:242)
-        if np.linalg.cond(np.eye(self.Nx) - A) > 1e12:
-            raise NotImplementedError("TargetSelector on the GPU eliminates xs through (I - A)^-1: A must not have an "
-                                      "eigenvalue at 1 (an integrating plant needs H to pin the target)")
         self._setup_fixed_matrices()
         self._dev = _device_index(device)
         self._handle = None
@@ -150,6 +149,10 @@ class TargetSelector:
         self.tb = np.block([[np.zeros((nx, ny)), self.Bd], [self.H, -(self.H @ self.Cd)]])
         self.P = scipy.linalg.block_diag(self.C.T @ (self.Qs @ self.C), self.Rs)
         ImA = np.eye(nx) - self.A
+        self.reduced = self.Nz != 0 or np.linalg.cond(ImA) > 1e12
+        if self.reduced:
+            self._setup_reduction()
+            return
         self.Gx = np.linalg.solve(ImA, self.B)
         self.Gd = np.linalg.solve(ImA, self.Bd)
         CG = self.C @ self.Gx
@@ -170,9 +173,72 @@ class TargetSelector:
             self.Mbar = 0.5 * (Mb + Mb.T)
             self.Ryd = self.C @ self.Gd + self.Cd
 
+    def _setup_reduction(self):
+        """Null-space reduction of ``tA w = tb s`` (w = [xs; us], s = [ysp; dhat]) for ``H`` non-empty or ``I - A``
+        singular, where xs cannot be eliminated through (I - A)^-1.
+
+        ``w = K s + Z v`` with ``K = tA^+ tb`` and ``Z`` an orthonormal basis of null(tA) (both from one SVD), so the
+        equalities hold for every ``v`` (``nw = Nu - Nz`` entries).  The reference objective becomes
+        ``1/2 v'(Z'PZ)v + f'v + const`` with ``f = Fy ysp + Fd dhat + f0``, and the inequalities become the ``mb`` rows
+        ``lo0 - R s <= Abar v <= hi0 - R s``: the output rows ``C Zx v`` with offset ``(C Kx + [0 Cd]) s`` when
+        output bounds are given, then the input rows ``Zu v`` with offset ``Ku s``.  The GPU kernel (csrc/ts.cu,
+        k_ts_general) solves that QP and reconstructs ``xs = Kx s + Zx v``, ``us = Ku s + Zu v``."""
+        nx, nu, ny, nd, nz = self.Nx, self.Nu, self.Ny, self.Nd, self.Nz
+        U, sv, Vt = np.linalg.svd(self.tA)
+        rank = int(np.sum(sv > max(self.tA.shape) * np.finfo(float).eps * sv[0]))
+        if rank < nx + nz:
+            raise ValueError(f"TargetSelector: tA = [I-A, -B; HC, 0] has rank {rank} < {nx + nz} rows: the target "
+                             "equalities are dependent or contradictory (uncontrollable integrator, or H rows that the "
+                             "inputs cannot move independently)")
+        self.nw = nu - nz
+        self.Z = Vt[rank:].T
+        self.K = Vt[:rank].T @ ((U.T @ self.tb) / sv[:, None])
+        self.Zx, self.Zu, self.Kx, self.Ku = self.Z[:nx], self.Z[nx:], self.K[:nx], self.K[nx:]
+        Hr = self.Z.T @ self.P @ self.Z
+        self.Hr = 0.5 * (Hr + Hr.T)
+        if self.nw:
+            ev = np.linalg.eigvalsh(self.Hr)
+            if not ev[0] > 1e-12 * ev[-1]:
+                raise ValueError(f"TargetSelector: the reduced Hessian Z'PZ is singular (eigenvalues {ev[0]:.3e} .. "
+                                 f"{ev[-1]:.3e}): the target is not unique; weight more outputs in Qs or the inputs in Rs")
+        # q(s) = [-C'Qs (ysp - Cd dhat); -Rs usp] (linearMPC.py:276-283) = Qsd s + q0
+        CQ = self.C.T @ self.Qs
+        Qsd = np.vstack([np.hstack([-CQ, CQ @ self.Cd]), np.zeros((nu, ny + nd))])
+        q0 = np.vstack([np.zeros((nx, 1)), -(self.Rs @ self.usp)])
+        Fs = self.Z.T @ (self.P @ self.K + Qsd)
+        self.Fy, self.Fd, self.f0 = Fs[:, :ny], Fs[:, ny:], self.Z.T @ q0
+        if self.ylb is not None and self.yub is not None:
+            Ry = self.C @ self.Kx + np.hstack([np.zeros((ny, ny)), self.Cd])
+            self.Abar = np.vstack([self.C @ self.Zx, self.Zu])
+            self.R = np.vstack([Ry, self.Ku])
+            self.lo0, self.hi0 = np.vstack([self.ylb, self.ulb]), np.vstack([self.yub, self.uub])
+        else:
+            self.Abar, self.R, self.lo0, self.hi0 = self.Zu, self.Ku, self.ulb, self.uub
+        self.mb = self.Abar.shape[0]
+        if self.mb > 160:
+            raise NotImplementedError(f"TargetSelector: {self.mb} constraint rows (Ny + Nu with output bounds) exceed "
+                                      "the 160 the GPU solver holds per sample")
+        if self.nw:
+            cho = scipy.linalg.cho_factor(self.Hr)
+            self.Hinv = scipy.linalg.cho_solve(cho, np.eye(self.nw))
+            self.Hinv = 0.5 * (self.Hinv + self.Hinv.T)
+            self.AH = scipy.linalg.cho_solve(cho, self.Abar.T).T
+        else:
+            self.Hinv, self.AH = np.zeros((0, 0)), np.zeros((self.mb, 0))
+        Mb = self.AH @ self.Abar.T
+        self.Mbar = 0.5 * (Mb + Mb.T)
+
     def _create(self):
         L = _lib.lib()
         hnd = C.c_void_p()
+        if self.reduced:
+            arrs = [_lib.host(a) for a in (self.Hinv, self.Abar, self.AH, self.Mbar, self.Fy, self.Fd, self.f0, self.R,
+                                           self.lo0, self.hi0, self.Kx, self.Ku, self.Zx, self.Zu, self.ulb, self.uub)]
+            rc = L.nnmpc_ts_create_reduced(C.byref(hnd), self.Nx, self.Nu, self.Ny, self.Nd, self.nw, self.mb,
+                                           *[_lib.hptr(a) if a.size else None for a in arrs], self._dev)
+            _lib.check(rc, "nnmpc_ts_create_reduced")
+            self._handle = hnd
+            return
         arrs = [_lib.host(a) for a in (self.Ht, self.Fy, self.Fd if self.Nd else np.zeros((self.Nu, 1)), self.f0,
                                        self.Gx, self.Gd if self.Nd else np.zeros((self.Nx, 1)), self.ulb, self.uub)]
         rc = L.nnmpc_ts_create(C.byref(hnd), self.Nx, self.Nu, self.Ny, self.Nd, *[_lib.hptr(a) for a in arrs],
