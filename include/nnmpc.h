@@ -320,6 +320,33 @@ int nnmpc_oz_gemm_test(int M, int N, int K, const double* A, const double* Bt, d
 int nnmpc_exact_apply_test(int kind, int pipe, int variant, int B, int n, int nu, const double* Op, const int* rows,
                            const int* count, int max_rows, const double* A, const double* C, const double* lb,
                            const double* ub, double* X, unsigned long long* kres, void* stream);
+/* nnmpc_lp_step_test: one kernel of the mixed-precision iteration (the fp16 tensor-core pass and the FP64 kernels around
+ * it), called as the closed-loop engine calls it, on caller-owned device state; synchronises the stream.
+ *   op 0 split        T1 = fp16(s Top), T2 = fp16(s Top - T1), s = 2^(10 - e) for top_max = m 2^e (m in [0.5, 1)):
+ *                     D_out / S_out receive T1 / T2 as n rows of ldh = 64 ceil(n / 64) halves, sc_out[0] = s
+ *   op 1 anchor_prep  listed rows: W = 2 clip(V) - V, E = 0
+ *   op 2 dr_first     listed rows: one FP64 step from X, first increment into D_out at row pos_r[r] (none if < 0)
+ *   op 3 reanchor     listed rows in emit_state: X = Z, W = Z + W rinv (rinv per column)
+ *   op 4 emit         listed rows in emit_state: first increment from (X, W = w_lp) into D_out at row pos_r[r]
+ *   op 5 iterate      one tensor-core pass over operand rows [0, *len_r): reads D_in (and S_in), writes D_out and
+ *                     S_out at row pos_w[r] for r = list_r[p] in iter_state, folds max |d| into dres
+ *   op 6 correct      X += T2 S_in / (s sS) over the rows op 5 would take part with
+ * Listed rows (ops 1-4) are rows[p] for p < *count.  list_r, pos_w, pos_r NULL = identity; need2 (per 128 operand rows)
+ * and tile_stat[2] are nullable.  kernel (ops 5, 6): -1 = the process default (NNMPC_LP_KERNEL, NNMPC_LP_TILE,
+ * NNMPC_LP1_TILE), else two-term passes (s_mode 0) 0 = 128 x 128 tiles, 1 = 256 x 128 tiles, 2 = CTA pair, one-term
+ * passes (s_mode 1, 2) and op 6: 0 = 128 x 128, 1 = 256 x 128.  s_mode (ops 2, 4, 5): 0 = no pending sums (S_out, sS
+ * untouched), 1 = add the increment to S_in, 2 = start a new pending sum.  Shapes: X, V, W, Z, D_*, S_* are B x n
+ * (fp16 as bit patterns), E is B x n floats, sc_in, sc_out, sS, dres, state, it, dtrig are per row, lb, ub are B x nu,
+ * rinv has n entries; count and len_r are device ints.  Refuses n odd or <= 0, nu <= 0, and s_mode != 0 (or op 6) with
+ * kernel 2. */
+int nnmpc_lp_step_test(int op, int kernel, int s_mode, double alpha, int n, int nu, int B, const double* Top,
+                       double top_max, const int* rows, const int* count, const int* list_r, const int* len_r,
+                       const int* pos_w, const int* pos_r, int* state, int iter_state, int emit_state,
+                       unsigned char* need2, double* X, double* V, double* W, float* E, double* sc_in, double* sc_out,
+                       double* sS, unsigned long long* dres, int* it, const double* dtrig, const double* rinv,
+                       const double* Z, const double* lb, const double* ub, const unsigned short* D_in,
+                       const unsigned short* S_in, unsigned short* D_out, unsigned short* S_out,
+                       unsigned long long* tile_stat, void* stream);
 /* nnmpc_lp_pass_probe (tools/probes/lp_pass_split.py): one tensor-core pass over B x n synthetic state with the production
  * epilogue (ms[0]), with an epilogue that only drains TMEM (ms[1]) and with the production epilogue but no TMA loads / MMAs
  * (ms[2]: the epilogue alone); then the deferred-second-term form: the one-term pass (ms[3]) and the second-term delivery

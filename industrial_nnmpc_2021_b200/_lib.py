@@ -81,6 +81,8 @@ SIGNATURES = {
     "nnmpc_oz_gemm_test": (C.c_int, [C.c_int, C.c_int, C.c_int, vp, vp, vp, vp]),
     "nnmpc_exact_apply_test": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, C.c_int, vp,
                                          vp, vp, vp, vp, vp, vp]),
+    "nnmpc_lp_step_test": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_int, vp, C.c_double]
+                           + [vp] * 6 + [vp, C.c_int, C.c_int] + [vp] * 21),
     "nnmpc_gemm_tn": (C.c_int, [C.c_int, C.c_int, C.c_int, vp, C.c_longlong, vp, C.c_longlong, vp, C.c_longlong,
                                 vp, vp]),
 }

@@ -140,9 +140,12 @@ int lp_emit(const int* rows, const int* count, int max_rows, int* state, int emi
 int lp_iterate(const LpOperator* op, LpState* s, int B, const int* list_r, const int* len_r, const int* pos_w, double* V,
                const double* lb, const double* ub, const int* state, int iter_state, unsigned long long* dres, int nu,
                double alpha, int device, cudaStream_t st, const unsigned char* need2, unsigned long long* tile_stat,
-               int s_mode) {
+               int s_mode, int kernel) {
   if (B <= 0) return 0;
   if (s_mode && !s->defer2) return set_error(NNMPC_ERR_BADARG, "lp_iterate: pending-sum buffers were not allocated");
+  if (kernel < -1 || kernel > (s_mode ? 1 : 2)) return set_error(NNMPC_ERR_BADARG, "lp_iterate: no kernel %d for s_mode %d", kernel, s_mode);
+  const int k2 = kernel >= 0 ? kernel : (lp_use_pair() ? 2 : lp_tile_m256());
+  const int k1 = kernel >= 0 ? kernel : lp1_tile_m256();
   EpiDelta::Params ep{};
   ep.s_mode = s_mode;
   if (s_mode) { ep.Sc = s->S[s->cur].p; ep.Sn = s->S[s->cur ^ 1].p; ep.sS = s->sS.p; }
@@ -150,7 +153,7 @@ int lp_iterate(const LpOperator* op, LpState* s, int B, const int* list_r, const
   ep.state = state; ep.iter_state = iter_state; ep.list_r = list_r; ep.pos_w = pos_w; ep.sc_in = s->sc_in.p; ep.sc_out = s->sc_out.p; ep.dres = dres;
   ep.n = s->n; ep.nu = nu; ep.alpha = alpha; ep.inv_sT = 1.0 / op->scale;
   // column-tile groups of at most ~24 MB of operator (both fp16 terms) per group
-  const int bn_tile = lp_use_pair() ? lp::BN2 : LpTileN128::BN;
+  const int bn_tile = k2 == 2 ? lp::BN2 : LpTileN128::BN;
   const double tile_mb = 2.0 * bn_tile * (double)op->ldh * 2.0 / 1048576.0;
   int group_cols = (int)(24.0 / tile_mb);
   if (group_cols < 1) group_cols = 1;
@@ -158,7 +161,7 @@ int lp_iterate(const LpOperator* op, LpState* s, int B, const int* list_r, const
   if (s_mode) {      // one-term pass (the kernel never touches the second operator map)
     g.need2 = nullptr;
     g.group_cols = 2 * group_cols;        // one term: the same bytes of operator cover twice the column tiles
-    cudaError_t e1 = lp1_tile_m256()
+    cudaError_t e1 = k1 == 1
                          ? lp::launch_lp_gemm<LpTile1M256, EpiDelta>(s->tmD256[s->cur], op->tm1, op->tm1, g, ep, device_sm_count(device), st)
                          : lp::launch_lp_gemm<LpTile1N128, EpiDelta>(s->tmD[s->cur], op->tm1, op->tm1, g, ep, device_sm_count(device), st);
     count_launch();
@@ -166,9 +169,9 @@ int lp_iterate(const LpOperator* op, LpState* s, int B, const int* list_r, const
     s->cur ^= 1;
     return 0;
   }
-  cudaError_t e = lp_use_pair()
+  cudaError_t e = k2 == 2
                       ? lp::launch_lp_gemm_pair<EpiDelta>(s->tmD[s->cur], op->tm1, op->tm2, g, ep, device_sm_count(device), st)
-                  : lp_tile_m256()
+                  : k2 == 1
                       ? lp::launch_lp_gemm<LpTileM256, EpiDelta>(s->tmD256[s->cur], op->tm1, op->tm2, g, ep, device_sm_count(device), st)
                       : lp::launch_lp_gemm<LpTileN128, EpiDelta>(s->tmD[s->cur], op->tm1, op->tm2, g, ep, device_sm_count(device), st);
   count_launch();
@@ -178,15 +181,16 @@ int lp_iterate(const LpOperator* op, LpState* s, int B, const int* list_r, const
 }
 
 int lp_correct(const LpOperator* op, LpState* s, int B, const int* list_r, const int* len_r, const int* state,
-               int iter_state, int device, cudaStream_t st, unsigned long long* tile_stat) {
+               int iter_state, int device, cudaStream_t st, unsigned long long* tile_stat, int kernel) {
   if (B <= 0) return 0;
   if (!s->defer2) return set_error(NNMPC_ERR_BADARG, "lp_correct: pending-sum buffers were not allocated");
+  if (kernel < -1 || kernel > 1) return set_error(NNMPC_ERR_BADARG, "lp_correct: no kernel %d", kernel);
   EpiAddX::Params ep{s->X.p, state, iter_state, list_r, s->sS.p, s->n, 1.0 / op->scale};
   const double tile_mb = LpTile1N128::BN * (double)op->ldh * 2.0 / 1048576.0;
   int group_cols = (int)(24.0 / tile_mb);
   if (group_cols < 1) group_cols = 1;
   lp::LpShape g{B, s->n, s->n, len_r, group_cols, nullptr, tile_stat, 0, 0};
-  cudaError_t e = lp1_tile_m256()
+  cudaError_t e = (kernel >= 0 ? kernel : lp1_tile_m256()) == 1
                       ? lp::launch_lp_gemm<LpTile1M256, EpiAddX>(s->tmS256[s->cur], op->tm2, op->tm2, g, ep, device_sm_count(device), st)
                       : lp::launch_lp_gemm<LpTile1N128, EpiAddX>(s->tmS[s->cur], op->tm2, op->tm2, g, ep, device_sm_count(device), st);
   count_launch();
@@ -225,6 +229,81 @@ __global__ void k_to_half(const double* __restrict__ A, long long rows, int cols
     const int c = (int)(i - r * ld);
     H[i] = __double2half(c < cols ? A[r * cols + c] : 0.0);
   }
+}
+
+enum { LP_SPLIT, LP_ANCHOR_PREP, LP_DR_FIRST, LP_REANCHOR, LP_EMIT, LP_ITERATE, LP_CORRECT };
+
+static int copy_rows_f16(void* dst, size_t dpitch, const void* src, size_t spitch, int n, int B, cudaStream_t st) {
+  if (!dst || !src) return 0;
+  NNMPC_CUDA(cudaMemcpy2DAsync(dst, dpitch, src, spitch, (size_t)n * sizeof(__half), (size_t)B, cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+template <class T>
+static int copy_n(T* dst, const T* src, size_t count, cudaStream_t st) {
+  if (!dst || !src) return 0;
+  NNMPC_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(T), cudaMemcpyDeviceToDevice, st));
+  return 0;
+}
+
+static int lp_step_run(int op, int kernel, int s_mode, double alpha, int n, int nu, int B, const double* Top,
+                       double top_max, const int* rows, const int* count, const int* list_r, const int* len_r,
+                       const int* pos_w, const int* pos_r, int* state, int iter_state, int emit_state,
+                       unsigned char* need2, double* X, double* V, double* W, float* E, double* sc_in, double* sc_out,
+                       double* sS, unsigned long long* dres, int* it, const double* dtrig, const double* rinv,
+                       const double* Z, const double* lb, const double* ub, const __half* D_in, const __half* S_in,
+                       __half* D_out, __half* S_out, unsigned long long* tile_stat, LpState& ls, LpOperator& lo,
+                       cudaStream_t st) {
+  int dev = 0;
+  NNMPC_CUDA(cudaGetDevice(&dev));
+  if (op == LP_SPLIT || op == LP_ITERATE || op == LP_CORRECT) NNMPC_TRY(lp_split_operator(Top, n, top_max, &lo, st));
+  if (op == LP_SPLIT) {
+    NNMPC_TRY(copy_rows_f16(D_out, lo.ldh * sizeof(__half), lo.T1.p, lo.ldh * sizeof(__half), (int)lo.ldh, n, st));
+    NNMPC_TRY(copy_rows_f16(S_out, lo.ldh * sizeof(__half), lo.T2.p, lo.ldh * sizeof(__half), (int)lo.ldh, n, st));
+    NNMPC_CUDA(cudaMemcpyAsync(sc_out, &lo.scale, sizeof(double), cudaMemcpyHostToDevice, st));
+    return 0;
+  }
+  ls.defer2 = s_mode != 0 || op == LP_CORRECT;
+  NNMPC_TRY(lp_state_ensure(&ls, B, n, st));
+  const size_t bn = (size_t)B * n, dp = (size_t)ls.ldd * sizeof(__half), sp = (size_t)n * sizeof(__half);
+  const bool wl = op == LP_REANCHOR || op == LP_EMIT;     // W is the state's Wl (else the caller's own buffer)
+  NNMPC_TRY(copy_n(ls.X.p, X, bn, st));
+  NNMPC_TRY(copy_n(ls.E.p, E, bn, st));
+  if (wl) NNMPC_TRY(copy_n(ls.Wl.p, W, bn, st));
+  NNMPC_TRY(copy_n(ls.sc_in.p, sc_in, (size_t)B, st));
+  NNMPC_TRY(copy_n(ls.sc_out.p, sc_out, (size_t)B, st));
+  if (ls.defer2) NNMPC_TRY(copy_n(ls.sS.p, sS, (size_t)B, st));
+  const int wr = op == LP_ITERATE ? 1 : 0;                 // buffer the op writes (it reads buffer 0)
+  if (op == LP_ITERATE || op == LP_CORRECT) {
+    NNMPC_TRY(copy_rows_f16(ls.D[0].p, dp, D_in, sp, n, B, st));
+    if (ls.defer2) NNMPC_TRY(copy_rows_f16(ls.S[0].p, dp, S_in, sp, n, B, st));
+  }
+  NNMPC_TRY(copy_rows_f16(ls.D[wr].p, dp, D_out, sp, n, B, st));
+  if (ls.defer2) NNMPC_TRY(copy_rows_f16(ls.S[wr].p, dp, S_out, sp, n, B, st));
+  ls.cur = 0;
+  switch (op) {
+    case LP_ANCHOR_PREP: NNMPC_TRY(lp_anchor_prep(rows, count, B, V, W, &ls, lb, ub, nu, st)); break;
+    case LP_DR_FIRST:
+      NNMPC_TRY(lp_dr_first(rows, count, B, &ls, V, W, lb, ub, state, it, iter_state, nu, alpha, pos_r, st, need2));
+      break;
+    case LP_REANCHOR: NNMPC_TRY(lp_reanchor(rows, count, B, state, emit_state, Z, rinv, &ls, st)); break;
+    case LP_EMIT:
+      NNMPC_TRY(lp_emit(rows, count, B, state, emit_state, iter_state, &ls, V, lb, ub, dtrig, nu, alpha, pos_r, st, need2));
+      break;
+    case LP_ITERATE:
+      NNMPC_TRY(lp_iterate(&lo, &ls, B, list_r, len_r, pos_w, V, lb, ub, state, iter_state, dres, nu, alpha, dev, st,
+                           need2, tile_stat, s_mode, kernel));
+      break;
+    default: NNMPC_TRY(lp_correct(&lo, &ls, B, list_r, len_r, state, iter_state, dev, st, tile_stat, kernel)); break;
+  }
+  NNMPC_TRY(copy_n(X, (const double*)ls.X.p, bn, st));
+  NNMPC_TRY(copy_n(E, (const float*)ls.E.p, bn, st));
+  if (wl) NNMPC_TRY(copy_n(W, (const double*)ls.Wl.p, bn, st));
+  NNMPC_TRY(copy_n(sc_in, (const double*)ls.sc_in.p, (size_t)B, st));
+  NNMPC_TRY(copy_n(sc_out, (const double*)ls.sc_out.p, (size_t)B, st));
+  if (ls.defer2) NNMPC_TRY(copy_n(sS, (const double*)ls.sS.p, (size_t)B, st));
+  NNMPC_TRY(copy_rows_f16(D_out, sp, ls.D[wr].p, dp, n, B, st));
+  if (ls.defer2) NNMPC_TRY(copy_rows_f16(S_out, sp, ls.S[wr].p, dp, n, B, st));
+  return 0;
 }
 
 }  // namespace nnmpc
@@ -269,6 +348,52 @@ int nnmpc_lp_gemm_test(int M, int N, int K, const double* A, const double* Bt, d
   Ah.release();
   op.T1.release();
   op.T2.release();
+  return rc;
+}
+
+// Self test of the mixed-precision iteration as the engine calls it (include/nnmpc.h).  The caller's state is copied
+// into an LpState / LpOperator sized for B rows (padded, TMA-mapped, padding zero); the operand buffer an op writes is
+// pre-loaded from D_out / S_out, so positions it must not write come back as the caller left them.
+int nnmpc_lp_step_test(int op, int kernel, int s_mode, double alpha, int n, int nu, int B, const double* Top,
+                       double top_max, const int* rows, const int* count, const int* list_r, const int* len_r,
+                       const int* pos_w, const int* pos_r, int* state, int iter_state, int emit_state,
+                       unsigned char* need2, double* X, double* V, double* W, float* E, double* sc_in, double* sc_out,
+                       double* sS, unsigned long long* dres, int* it, const double* dtrig, const double* rinv,
+                       const double* Z, const double* lb, const double* ub, const unsigned short* D_in,
+                       const unsigned short* S_in, unsigned short* D_out, unsigned short* S_out,
+                       unsigned long long* tile_stat, void* stream) {
+  if (op < LP_SPLIT || op > LP_CORRECT || n <= 0 || (n & 1) || nu <= 0 || B <= 0 || s_mode < 0 || s_mode > 2 ||
+      kernel < -1 || kernel > 2)
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_lp_step_test: bad op, kernel, s_mode or shape (n must be even and > 0, nu > 0)");
+  if ((s_mode != 0 || op == LP_CORRECT) && kernel == 2)
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_lp_step_test: the CTA-pair kernel has no one-term form");
+  const bool listed = op != LP_SPLIT && op != LP_ITERATE && op != LP_CORRECT;
+  const bool defer = s_mode != 0 && (op == LP_DR_FIRST || op == LP_EMIT || op == LP_ITERATE);
+  bool ok = true;
+  switch (op) {
+    case LP_SPLIT: ok = Top && D_out && S_out && sc_out; break;
+    case LP_ANCHOR_PREP: ok = V && W && E && lb && ub; break;
+    case LP_DR_FIRST: ok = X && V && W && E && lb && ub && sc_in && sc_out && state && it && D_out; break;
+    case LP_REANCHOR: ok = state && Z && W && rinv && X; break;
+    case LP_EMIT: ok = state && V && W && E && D_out && lb && ub && sc_in && sc_out && dtrig; break;
+    case LP_ITERATE: ok = Top && len_r && X && V && E && lb && ub && state && dres && sc_in && sc_out && D_in && D_out &&
+                          (s_mode != 1 || S_in); break;
+    default: ok = Top && len_r && state && X && S_in && sS; break;
+  }
+  if (!ok || (listed && (!rows || !count)) || (defer && (!S_out || !sS)))
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_lp_step_test: a buffer the op needs is missing");
+  cudaStream_t st = (cudaStream_t)stream;
+  LpState ls;
+  LpOperator lo;
+  int rc = lp_step_run(op, kernel, s_mode, alpha, n, nu, B, Top, top_max, rows, count, list_r, len_r, pos_w, pos_r,
+                       state, iter_state, emit_state, need2, X, V, W, E, sc_in, sc_out, sS, dres, it, dtrig, rinv, Z,
+                       lb, ub, reinterpret_cast<const __half*>(D_in), reinterpret_cast<const __half*>(S_in),
+                       reinterpret_cast<__half*>(D_out), reinterpret_cast<__half*>(S_out), tile_stat, ls, lo, st);
+  if (rc == 0 && cudaStreamSynchronize(st) != cudaSuccess)
+    rc = set_error(NNMPC_ERR_CUDA, "nnmpc_lp_step_test: %s", cudaGetErrorString(cudaGetLastError()));
+  cudaStreamSynchronize(st);
+  ls.release();
+  lo.release();
   return rc;
 }
 

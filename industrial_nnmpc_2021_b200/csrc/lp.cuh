@@ -56,7 +56,8 @@ int lp_anchor_prep(const int* rows, const int* count, int max_rows, const double
 int lp_anchor_gemm(const int* rows, const int* count, int max_rows, const double* W, const double* Top, const double* C,
                    double* X, int n, cudaStream_t st);
 // listed rows: one FP64 Douglas-Rachford step from the exact x, first fp16 increment, state := iter_state
-// pos_r: sample row -> row of the operand buffer the next pass reads (null = identity)
+// pos_r: sample row -> row of the operand buffer the next pass reads (null = identity); a negative position writes no
+// operand row (no D, S or need2 flag; E, the scales, state and it are updated)
 int lp_dr_first(const int* rows, const int* count, int max_rows, LpState* s, double* V, double* W, const double* lb,
                 const double* ub, int* state, int* it, int iter_state, int nu, double alpha, const int* pos_r,
                 cudaStream_t st, unsigned char* need2 = nullptr);   // need2: operand tiles of these rows get both operator terms
@@ -64,22 +65,31 @@ int lp_dr_first(const int* rows, const int* count, int max_rows, LpState* s, dou
 int lp_reanchor(const int* rows, const int* count, int max_rows, const int* state, int emit_state, const double* Z,
                 const double* rinv, LpState* s, cudaStream_t st);
 // listed rows in emit_state: first fp16 increment from the exactly anchored (x, w_lp); state := iter_state
+// (pos_r as for lp_dr_first, a negative position included)
 int lp_emit(const int* rows, const int* count, int max_rows, int* state, int emit_state, int iter_state, LpState* s,
             const double* V, const double* lb, const double* ub, const double* dtrig, int nu, double alpha,
             const int* pos_r, cudaStream_t st, unsigned char* need2 = nullptr);
 // One tensor-core pass over the operand rows [0, *len_r) (at most B); flips s->cur.  Operand row p belongs to
 // sample list_r[p]; it takes part iff state[sample] == iter_state, and its next increment is written to
 // operand row pos_w[sample] of the other buffer (so the layout is re-compacted one pass behind the live list).
+// Precondition: 0 <= pos_w[sample] < B for every sample that takes part (the epilogue does not check it).  The engine
+// (sim.cu) meets it, and passes non-negative positions to lp_dr_first / lp_emit as well: k_step gives every live row
+// (ITER, RENEW, ANCHOR, EMIT) a position and -1 only to IDLE rows, a row is IDLE only when no chunk is left for its slot,
+// and an IDLE row never becomes live again; the rows of one layout that iterate, start a QP (anchor) or are re-emitted
+// before the next k_step were live when it was built.
+// kernel: -1 = the process default (NNMPC_LP_KERNEL, NNMPC_LP_TILE; NNMPC_LP1_TILE for s_mode != 0), else s_mode 0:
+// 0 = 128 x 128 tiles, 1 = 256 x 128 tiles, 2 = CTA pair; s_mode 1 / 2: 0 = 128 x 128, 1 = 256 x 128.
 int lp_iterate(const LpOperator* op, LpState* s, int B, const int* list_r, const int* len_r, const int* pos_w, double* V,
                const double* lb, const double* ub, const int* state, int iter_state, unsigned long long* dres, int nu,
                double alpha, int device, cudaStream_t st, const unsigned char* need2 = nullptr,
-               unsigned long long* tile_stat = nullptr, int s_mode = 0);
+               unsigned long long* tile_stat = nullptr, int s_mode = 0, int kernel = -1);
 // Deferred second operator term: x += T2 S / (s_T sS) over the operand rows the NEXT lp_iterate will read (same
 // list / state predicate); that pass must then run with s_mode = 2 (a new pending sum starts).  s_mode of
 // lp_iterate: 0 = two-term pass (no pending sums), 1 = one-term pass, increment added to the pending sum, 2 = one-term
 // pass, pending sum restarted.
 int lp_correct(const LpOperator* op, LpState* s, int B, const int* list_r, const int* len_r, const int* state,
-               int iter_state, int device, cudaStream_t st, unsigned long long* tile_stat = nullptr);   // tile_stat[0] += tiles
+               int iter_state, int device, cudaStream_t st, unsigned long long* tile_stat = nullptr,   // tile_stat[0] += tiles
+               int kernel = -1);     // -1 = NNMPC_LP1_TILE, 0 = 128 x 128 tiles, 1 = 256 x 128 tiles
 
 
 }  // namespace nnmpc

@@ -167,8 +167,10 @@ struct EpiDelta {
     const __half q0 = quantise_dw_fast(dw0, ri.s_out, ri.inv_out, e.x);
     const __half q1 = quantise_dw_fast(dw1, ri.s_out, ri.inv_out, e.y);
     q = __halves2half2(q0, q1);
-    const float a = (float)((d0 <= d1) ? d1 : d0);       // NaN propagates
-    dm = (!valid || a <= dm) ? dm : a;                   // lanes that ran on a stand-in row must not touch the residual
+    // a NaN in d, or a non-finite residual e (v or E not finite while d is), makes the row's residual NaN (0 e = +-0
+    // otherwise, and a + +-0 = a for a >= 0: finite residuals are unchanged)
+    const float a = fmaf(0.f, e.x, fmaf(0.f, e.y, nan_max((float)d0, (float)d1)));
+    if (valid) dm = nan_max(dm, a);                      // lanes that ran on a stand-in row must not touch the residual
   }
 
   // ---- the chunk as a software pipeline over QUARTERS (QR = NI / 4 row iterations = 2 rows x 2 columns per lane) ----
@@ -331,8 +333,7 @@ struct EpiDelta {
       // the LPR lanes of a row group hold disjoint columns of the same rows; NaN must survive the reduction
 #pragma unroll
       for (int o = 1; o < LPR; o <<= 1) {
-        const float t = __shfl_xor_sync(0xffffffffu, m, o);
-        m = (t <= m) ? m : t;
+        m = nan_max(m, __shfl_xor_sync(0xffffffffu, m, o));
       }
       const int row = sm->info[rg + RG * i].row;
       if (cp == 0 && row >= 0) {
@@ -505,15 +506,13 @@ k_dr_first(const int* __restrict__ rows, const int* __restrict__ count, double* 
     dr_delta_one(x, v, W[s * n + j], l, u, alpha, dw, a);
     V[s * n + j] = v;
     W[s * n + j] = dw;                    // staged for the second pass
-    dmax = (a <= dmax) ? dmax : a;
-    const double b = fabs(dw);
-    wmax = (b <= wmax) ? wmax : b;
+    dmax = nan_max(dmax, a);
+    wmax = nan_max(wmax, fabs(dw));
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
-    const double a = __shfl_xor_sync(0xffffffffu, dmax, o), b = __shfl_xor_sync(0xffffffffu, wmax, o);
-    dmax = (a <= dmax) ? dmax : a;
-    wmax = (b <= wmax) ? wmax : b;
+    dmax = nan_max(dmax, __shfl_xor_sync(0xffffffffu, dmax, o));
+    wmax = nan_max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
   }
   if ((threadIdx.x & 31) == 0) {
     red[0][threadIdx.x >> 5] = dmax;
@@ -523,16 +522,16 @@ k_dr_first(const int* __restrict__ rows, const int* __restrict__ count, double* 
   dmax = red[0][0];
   wmax = red[1][0];
   for (int w = 1; w < 8; ++w) {
-    dmax = (red[0][w] <= dmax) ? dmax : red[0][w];
-    wmax = (red[1][w] <= wmax) ? wmax : red[1][w];
+    dmax = nan_max(dmax, red[0][w]);
+    wmax = nan_max(wmax, red[1][w]);
   }
   const double sq = pow2_scale(wmax), inv = 1.0 / sq;
   const long long dpos = pos_r ? pos_r[s] : s;      // row of the operand buffer the next pass reads for this sample
   for (int j = threadIdx.x; j < n; j += blockDim.x) {
     float e;
     const __half q = quantise_dw(W[s * n + j], sq, inv, e);
-    D[dpos * ldd + j] = q;
-    if (S) S[dpos * ldd + j] = __float2half_rn(0.125f * __half2float(q));    // deferred second term: the pending sum starts
+    if (dpos >= 0) D[dpos * ldd + j] = q;
+    if (S && dpos >= 0) S[dpos * ldd + j] = __float2half_rn(0.125f * __half2float(q));    // deferred second term: the pending sum starts
     E[s * n + j] = e;
   }
   if (threadIdx.x == 0) {
@@ -591,18 +590,14 @@ k_lp_emit(const int* __restrict__ rows, const int* __restrict__ count, int* __re
     const double z = clipd(v, lb[s * nu + k], ub[s * nu + k]);
     const double dw = (2.0 * z - v) - WL[s * n + j];
     WL[s * n + j] = dw;                   // staged for the second pass
-    const double b = fabs(dw);
-    wmax = (b <= wmax) ? wmax : b;
+    wmax = nan_max(wmax, fabs(dw));
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const double b = __shfl_xor_sync(0xffffffffu, wmax, o);
-    wmax = (b <= wmax) ? wmax : b;
-  }
+  for (int o = 16; o > 0; o >>= 1) wmax = nan_max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = wmax;
   __syncthreads();
   wmax = red[0];
-  for (int w = 1; w < 8; ++w) wmax = (red[w] <= wmax) ? wmax : red[w];
+  for (int w = 1; w < 8; ++w) wmax = nan_max(wmax, red[w]);
   const double sq = pow2_scale(wmax), inv = 1.0 / sq;
   const long long dpos = pos_r ? pos_r[s] : s;      // row of the operand buffer the next pass reads for this sample
   for (int j = threadIdx.x; j < n; j += blockDim.x) {

@@ -56,6 +56,16 @@ __device__ __forceinline__ float row_max_keep_nan(float m, float h) {
   return (m != m || h != h) ? __int_as_float(0x7fffffff) : fmaxf(m, h);
 }
 
+// running maximum that keeps a NaN wherever it meets one ((b <= m) ? m : b alone drops an m that is NaN); the same
+// value as (b <= m) ? m : b whenever neither operand is NaN
+__device__ __forceinline__ double nan_max(double m, double b) { return (b <= m || m != m) ? m : b; }
+// fp32: one max.NaN instruction (a NaN operand gives NaN); the epilogue of the tensor-core pass is bound by issue
+__device__ __forceinline__ float nan_max(float m, float b) {
+  float r;
+  asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(m), "f"(b));
+  return r;
+}
+
 // clip in the reference's order (np.where(u > ub, ub, u), then np.where(u < lb, lb, u)): a NaN stays NaN
 __device__ __forceinline__ double clip_keep_nan(double v, double lb, double ub) {
   v = v > ub ? ub : v;

@@ -423,14 +423,14 @@ k_oz_pack_network_input(const double* __restrict__ x, const double* __restrict__
       double v1, v2;
       value(c, v1, v2);
       const double a1 = fabs(v1), a2 = fabs(v2);
-      m1 = oz::nan_max(m1, a1);
-      m2 = oz::nan_max(m2, a2);
+      m1 = nan_max(m1, a1);
+      m2 = nan_max(m2, a2);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       const double a1 = __shfl_xor_sync(0xffffffffu, m1, o), a2 = __shfl_xor_sync(0xffffffffu, m2, o);
-      m1 = oz::nan_max(m1, a1);
-      m2 = oz::nan_max(m2, a2);
+      m1 = nan_max(m1, a1);
+      m2 = nan_max(m2, a2);
     }
     double inv[2], fs[2];
     const double mm[2] = {m1, m2};

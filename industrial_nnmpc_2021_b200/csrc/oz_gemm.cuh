@@ -24,6 +24,7 @@
 //   warps 2-5  epilogue: tcgen05.ld the int32 levels of the warp's 32 rows, fold them in FP64 from the
 //              smallest level up, scale by 2^(f+e), hand 16-column row chunks to the fused epilogue functor
 #pragma once
+#include "nnmpc_common.cuh"
 #include "lp_gemm.cuh"   // PTX wrappers shared with the fp16 kernel (mbarrier, TMA, TMEM, descriptors)
 
 namespace nnmpc {
@@ -556,9 +557,6 @@ inline cudaError_t launch_oz_gemm2(const CUtensorMap& tmA, const CUtensorMap& tm
   oz_gemm2_kernel<LLO, LHI, BN_, Epi><<<grid, THREADS2, T::SMEM_BYTES, st>>>(tmA, tmB, g, ep);
   return cudaGetLastError();
 }
-
-// max of |row| entries that keeps a NaN wherever it meets one ((b <= m) ? m : b alone drops an m that is NaN)
-__device__ __forceinline__ double nan_max(double m, double b) { return (b <= m || m != m) ? m : b; }
 
 // ---- slicing: one CTA per row; rows[] (optional) gathers the source rows, position p is the destination row -----
 //   src row -> 2^f (max |a| <= 2^(f-1)) and NS signed base-128 digit planes dst[(s * rows_pad + p) * ldb + k]
