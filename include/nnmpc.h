@@ -76,6 +76,25 @@ int nnmpc_prof_readn(int nchan, double* ms, double* flops, long long* launches, 
 int nnmpc_qp_create(nnmpc_qp_t** out, int n, int nxa, int nu, int N,
                     const double* P_host, const double* tq_host, const double* Top_host,
                     const double* Mtq_host, const double* Kunc_host, double alpha, int device);
+/* Regulator of a re-parameterised (open-loop unstable) plant, u = K x + v, solved in v by a primal-dual interior-point
+ * method (Mehrotra predictor-corrector, one Riccati recursion per Newton step; industrial_nnmpc_2021_b200/csrc/ipm.cu)
+ * on the stagewise form of the reference's general-G QP (lib/linearMPC.py:366-382, :476-493):
+ *   min 1/2 sum_{k<N} (x_k'Q x_k + v_k'R v_k + 2 x_k'M v_k) + 1/2 x_N'Pf x_N
+ *   s.t. x_{k+1} = A x_k + B v_k,  x_0 = x0,  lb <= K x_k + v_k <= ub      (A = A_open + B K stable)
+ * Host arrays, row-major, padded with zeros to nxa_ld states: A, Q, Pf nxa_ld x nxa_ld, B, M nxa_ld x nu, R nu x nu,
+ * K nu x nxa_ld.  nxa_ld <= 64 and nu <= 32 (NNMPC_ERR_UNSUPPORTED otherwise).  The handle is an ordinary regulator:
+ * nnmpc_qp_solve[_host], nnmpc_online_run and nnmpc_sim_* accept it.  Through it u = K x + v along the forward roll-out
+ * (the reference's output, :507-509); v_state / warm are ignored (every solve starts cold); kkt is the relative KKT
+ * certificate of ipm.cu at the returned point; cost is the reference's objective 1/2 v'Pv + (tq x0)'v (not the u-space
+ * value the Douglas-Rachford path reports); iters counts interior-point iterations.  A sample with lb >= ub somewhere,
+ * a NaN bound or a non-finite x0 returns NaN with iters = max_iter (NNMPC_WARN_MAXITER); a bound at +-Inf is absent.
+ * nnmpc_qp_set_penalty refuses the handle (NNMPC_ERR_BADARG).  nnmpc_sim_create builds a lock-step engine on it
+ * (per step: target selector, interior-point QPs, dataset rows and plant step over the whole batch); the precision,
+ * slots, cadence, tail, exact-GEMM, one-term and second-term setters are accepted and have no effect, and
+ * nnmpc_sim_stats reports interior-point iterations as row-iterations. */
+int nnmpc_qp_create_ipm(nnmpc_qp_t** out, int nxa_ld, int nu, int N, const double* A_host, const double* B_host,
+                        const double* Q_host, const double* R_host, const double* M_host, const double* Pf_host,
+                        const double* K_host, int device);
 /* The ADMM penalty vector rho (host, n doubles, all > 0) behind Top = (P + diag(rho))^-1 diag(rho).  Needed by the
  * mixed-precision closed loop (nnmpc_sim_set_precision), which re-anchors x = Top w - c from the exact gradient
  * g = P z + q of its KKT checks:  w := z + g / rho  gives  x = z  exactly. */

@@ -32,6 +32,7 @@ SIGNATURES = {
     "nnmpc_prof_readn": (C.c_int, [C.c_int, c_double_p, c_double_p, C.POINTER(C.c_longlong), C.c_int]),
     "nnmpc_qp_create": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp,
                                   C.c_double, C.c_int]),
+    "nnmpc_qp_create_ipm": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp, vp, C.c_int]),
     "nnmpc_qp_set_penalty": (C.c_int, [vp, vp]),
     "nnmpc_qp_destroy": (C.c_int, [vp]),
     "nnmpc_qp_solve": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, vp, C.c_int, vp, vp, vp, C.c_double, C.c_int, vp]),

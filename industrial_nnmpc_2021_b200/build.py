@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libnnmpc.so")
-SOURCES = ["qp.cu", "ts.cu", "sim.cu", "mlp.cu", "gemm_bench.cu", "lp.cu", "oz.cu", "online.cu"]
+SOURCES = ["qp.cu", "ts.cu", "sim.cu", "mlp.cu", "gemm_bench.cu", "lp.cu", "oz.cu", "online.cu", "ipm.cu"]
 HEADERS = ["gemm_f64.cuh", "nnmpc_common.cuh", "qp.cuh", "ts.cuh", "lp.cuh", "lp_gemm.cuh", "lp_iter.cuh", "oz.cuh", "oz_gemm.cuh", "mlp_tc.cuh", os.path.join("..", "..", "include", "nnmpc.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--use_fast_math=false"]

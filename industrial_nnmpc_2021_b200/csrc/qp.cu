@@ -146,6 +146,7 @@ int qp_solve_device(nnmpc_qp* h, int B, const double* x0, const double* lb, cons
                     double* v_state, int warm, QpOutputs out, double tol, int max_iter, cudaStream_t st,
                     long long* iter_sum_out) {
   if (B <= 0) return 0;
+  if (h->ipm) return ipm_solve_device(h, B, x0, lb, ub, u, out, tol, max_iter, st, iter_sum_out);
   if (max_iter < 1) max_iter = 1;
   NNMPC_TRY(qp_ensure_scratch(h, B));
   const int n = h->n, nu = h->nu, nxa = h->nxa;
@@ -336,6 +337,9 @@ int nnmpc_qp_create(nnmpc_qp_t** out, int n, int nxa, int nu, int N, const doubl
 
 int nnmpc_qp_set_penalty(nnmpc_qp_t* h, const double* rho_host) {
   if (!h || !rho_host) return set_error(NNMPC_ERR_BADARG, "nnmpc_qp_set_penalty: null argument");
+  if (h->ipm)
+    return set_error(NNMPC_ERR_BADARG, "nnmpc_qp_set_penalty: this handle solves by interior point (nnmpc_qp_create_ipm) "
+                     "and has no ADMM penalty");
   DeviceGuard dg(h->device);
   double* tmp = new (std::nothrow) double[(size_t)h->n];
   if (!tmp) return set_error(NNMPC_ERR_NOMEM, "out of host memory");
@@ -362,7 +366,7 @@ int nnmpc_qp_destroy(nnmpc_qp_t* h) {
   if (!h) return 0;
   DeviceGuard dg(h->device);
   if (h->rinv) cudaFree(h->rinv);
-  for (double* p : {h->P, h->Top, h->tq, h->Mtq, h->Kunc})
+  for (double* p : {h->P, h->Top, h->tq, h->Mtq, h->Kunc, h->iA, h->iB, h->iQ, h->iR, h->iM, h->iPf, h->iK, h->iAo, h->iQo, h->iMo})
     if (p) cudaFree(p);
   if (h->counts) cudaFree(h->counts);
   if (h->iter_sum) cudaFree(h->iter_sum);
@@ -374,6 +378,7 @@ int nnmpc_qp_destroy(nnmpc_qp_t* h) {
   h->lpop.release();
   h->ozP.release();
   h->ozTop.release();
+  h->ipm_scr.release();
   delete h;
   return 0;
 }

@@ -255,6 +255,9 @@ struct QpOutputs {
 int qp_solve_device(nnmpc_qp* h, int B, const double* x0, const double* lb, const double* ub, double* u,
                     double* v_state, int warm, QpOutputs out, double tol, int max_iter, cudaStream_t st,
                     long long* iter_sum_out);
+// the interior-point solver of a handle made by nnmpc_qp_create_ipm (ipm.cu); qp_solve_device dispatches to it
+int ipm_solve_device(nnmpc_qp* h, int B, const double* x0, const double* lb, const double* ub, double* u,
+                     QpOutputs out, double tol, int max_iter, cudaStream_t st, long long* iter_sum_out);
 
 // live timing of the iteration GEMM (bench.py roofline); spans are recorded only while enabled
 // channel 0: the iteration passes (FP64 DMMA GEMM, or the tcgen05 pass in mixed mode);
@@ -298,4 +301,9 @@ struct nnmpc_qp {
   // host-buffer staging for *_host entry points
   nnmpc::DevBuf<double> hx0, hlb, hub, hu, hcost, hkkt;
   nnmpc::DevBuf<int> hiters;
+  // nnmpc_qp_create_ipm: stagewise v-space operators of the interior-point solver (ipm.cu) instead of P, Top, ...
+  int ipm = 0;
+  double *iA = nullptr, *iB = nullptr, *iQ = nullptr, *iR = nullptr, *iM = nullptr, *iPf = nullptr, *iK = nullptr;
+  double *iAo = nullptr, *iQo = nullptr, *iMo = nullptr;   // the stage in the original inputs (Newton-step factorisation)
+  nnmpc::DevBuf<double> ipm_scr;      // per-CTA Riccati factors and iterates
 };

@@ -750,11 +750,115 @@ static int sim_ensure(nnmpc_sim* h, long long B) {
   return 0;
 }
 
+// ---- lock-step engine of an interior-point regulator handle (nnmpc_qp_create_ipm) ------------------------------------
+// The continuously batched engine above is built on Douglas-Rachford internals (operand buffers, anchors, per-row
+// triggers).  With an interior-point regulator every step runs over the whole batch, as the online loop does:
+//     target selector (fused regulator inputs) -> interior-point QPs (ipm.cu) -> dataset rows and plant step.
+// Precision, slots, cadence, tail, exact-GEMM and second-term options have no effect on it.
+
+// one CTA per trajectory: u = first move + target, dataset row, uprev, optional capture, x+ = [A|B|Bd][x|u|d]
+__global__ void __launch_bounds__(128)
+k_ipm_plant(int B, int T, int t, const double* __restrict__ U, int n, const double* __restrict__ us,
+            double* __restrict__ xcur, double* __restrict__ upcur, const double* __restrict__ dist,
+            double* __restrict__ row_u, const double* __restrict__ ABd, int nx, int nu, int nd, int kin_ld,
+            double* __restrict__ cap_useq) {
+  extern __shared__ double kin[];   // kin_ld
+  for (int s = blockIdx.x; s < B; s += gridDim.x) {
+    const long long o = (long long)s * T + t;
+    for (int c = threadIdx.x; c < kin_ld; c += blockDim.x) {
+      double v = 0.0;
+      if (c < nx) {
+        v = xcur[(long long)s * nx + c];
+      } else if (c < nx + nu) {
+        const int k = c - nx;
+        v = U[(long long)s * n + k] + us[o * nu + k];
+        row_u[o * nu + k] = v;
+        upcur[(long long)s * nu + k] = v;
+      } else if (c < nx + nu + nd) {
+        v = dist[o * nd + (c - nx - nu)];
+      }
+      kin[c] = v;
+    }
+    if (cap_useq)
+      for (int j = threadIdx.x; j < n; j += blockDim.x) cap_useq[o * n + j] = U[(long long)s * n + j] + us[o * nu + (j % nu)];
+    __syncthreads();
+    for (int i = threadIdx.x; i < nx; i += blockDim.x) {
+      double a = 0.0;
+      for (int c = 0; c < kin_ld; ++c) a += ABd[(long long)i * kin_ld + c] * kin[c];
+      xcur[(long long)s * nx + i] = a;
+    }
+    __syncthreads();
+  }
+}
+
+static int sim_run_ipm(nnmpc_sim* h, int B, int T, double* x_io, double* uprev_io, const double* sp, const double* dist,
+                       double* ox, double* ouprev, double* oxs, double* ous, double* ou, int* oiters, double* okkt,
+                       double tol, int max_iter, cudaStream_t st, const QpBatch* qb) {
+  nnmpc_qp* q = h->qp;
+  long long isum = 0;
+  int warn = 0;
+  if (qb) {
+    warn = ipm_solve_device(q, B, qb->X0, qb->LB, qb->UB, qb->U, QpOutputs{qb->cost, okkt, oiters, 1}, tol, max_iter, st,
+                            &isum);
+    if (warn < 0) return warn;
+  } else {
+    const int nx = h->nx, nu = h->nu, nd = h->nd, ny = h->ny, n = q->n, nxa = h->nxa_ld;
+    const size_t b = (size_t)B;
+    NNMPC_TRY(h->x0.ensure(b * nxa));
+    NNMPC_TRY(h->lb.ensure(b * nu));
+    NNMPC_TRY(h->ub.ensure(b * nu));
+    NNMPC_TRY(h->us_prev.ensure(b * nu));
+    NNMPC_TRY(h->dus.ensure(b * nu));
+    NNMPC_TRY(h->xcur.ensure(b * nx));
+    NNMPC_TRY(h->upcur.ensure(b * nu));
+    NNMPC_TRY(h->Z.ensure(b * n));
+    NNMPC_CUDA(cudaMemsetAsync(h->counts, 0, N_COUNTERS * sizeof(int), st));
+    NNMPC_CUDA(cudaMemsetAsync(h->x0.p, 0, b * nxa * 8, st));   // padding column of x0
+    NNMPC_CUDA(cudaMemsetAsync(h->us_prev.p, 0, b * nu * 8, st));
+    NNMPC_CUDA(cudaMemcpyAsync(h->xcur.p, x_io, b * nx * 8, cudaMemcpyDeviceToDevice, st));
+    NNMPC_CUDA(cudaMemcpyAsync(h->upcur.p, uprev_io, b * nu * 8, cudaMemcpyDeviceToDevice, st));
+    const size_t smem = (size_t)h->kin_ld * sizeof(double);
+    if (smem > 48 * 1024) return set_error(NNMPC_ERR_UNSUPPORTED, "plant step: nx + nu + nd = %d is too large", h->kin_ld);
+    for (int t = 0; t < T; ++t) {
+      TsFused F{};
+      F.x = h->xcur.p; F.uprev = h->upcur.p; F.x0 = h->x0.p; F.nxa_ld = nxa; F.lb = h->lb.p; F.ub = h->ub.p;
+      F.us_prev = h->us_prev.p; F.dus = h->dus.p;
+      F.row_x = ox + (size_t)t * nx; F.row_uprev = ouprev + (size_t)t * nu;
+      F.row_stride_x = (long long)T * nx; F.row_stride_u = (long long)T * nu;
+      NNMPC_TRY(ts_solve_device(h->ts, B, sp + (size_t)t * ny, (long long)T * ny, dist + (size_t)t * nd, (long long)T * nd,
+                                oxs + (size_t)t * nx, (long long)T * nx, ous + (size_t)t * nu, (long long)T * nu, nullptr, 0,
+                                &F, nullptr, h->counts + F_TS_FAIL, st));
+      long long it = 0;
+      const int rc = ipm_solve_device(q, B, h->x0.p, h->lb.p, h->ub.p, h->Z.p,
+                                      QpOutputs{h->cap_cost ? h->cap_cost + t : nullptr, okkt ? okkt + t : nullptr,
+                                                oiters ? oiters + t : nullptr, T},
+                                      tol, max_iter, st, &it);
+      if (rc < 0) return rc;
+      warn |= rc;
+      isum += it;
+      k_ipm_plant<<<row_grid(B), 128, smem, st>>>(B, T, t, h->Z.p, n, ous, h->xcur.p, h->upcur.p, dist, ou, h->ABd, nx, nu, nd,
+                                                  h->kin_ld, h->cap_useq);
+      count_launch();
+    }
+    NNMPC_CUDA(cudaMemcpyAsync(x_io, h->xcur.p, b * nx * 8, cudaMemcpyDeviceToDevice, st));
+    NNMPC_CUDA(cudaMemcpyAsync(uprev_io, h->upcur.p, b * nu * 8, cudaMemcpyDeviceToDevice, st));
+    NNMPC_CUDA(cudaMemcpyAsync(h->pin, h->counts, N_COUNTERS * sizeof(int), cudaMemcpyDeviceToHost, st));
+    NNMPC_CUDA(cudaStreamSynchronize(st));
+    NNMPC_CUDA(cudaGetLastError());
+    if (h->pin[F_TS_FAIL]) warn |= NNMPC_WARN_TARGET;
+  }
+  h->tot_rowiters += isum;
+  h->tot_qps += (long long)B * (qb ? 1 : T);
+  return warn;
+}
+
 static int sim_run_device(nnmpc_sim* h, int Btot, int T, double* x_io, double* uprev_io, const double* sp,
                           const double* dist, double* ox, double* ouprev, double* oxs, double* ous, double* ou,
                           int* oiters, double* okkt, double tol, int max_iter, int resume, cudaStream_t st,
                           const QpBatch* qb = nullptr) {
   if (Btot <= 0 || T <= 0) return 0;
+  if (h->qp->ipm) return sim_run_ipm(h, Btot, T, x_io, uprev_io, sp, dist, ox, ouprev, oxs, ous, ou, oiters, okkt, tol, max_iter,
+                                     st, qb);
   if (max_iter < 1) max_iter = 1;
   // B trajectory slots advance concurrently; with more chunks than slots the rest queue up and a slot that
   // finishes its chunk takes the next one (cold start), so the batch stays full until the queue is empty

@@ -24,6 +24,7 @@ from .condense import dlqr, dlqe, c2d          # noqa: F401  (re-exported like t
 
 DEFAULT_TOL = 1e-9        # stop on true KKT residual ||u - clip(u - (Pu+q))||_inf <= tol
 DEFAULT_MAX_ITER = 20000
+IPM_MAX_ITER = 200        # interior-point regulators (solver == "ipm") when max_iter is left at its default
 
 
 def _torch():
@@ -313,6 +314,14 @@ class TargetSelector:
 
 
 # ------------------------------------------------------------------------------ regulator
+def _is_factorisation_error(exc):
+    """A failed Cholesky of the set-up (scipy / NumPy, or torch.linalg on the GPU set-up path)."""
+    if isinstance(exc, np.linalg.LinAlgError):
+        return True
+    torch = sys.modules.get("torch")
+    return torch is not None and isinstance(exc, torch.linalg.LinAlgError)
+
+
 class DenseQPRegulator:
     """Condensed regulator QP (linearMPC.py:321-517) with a batched GPU solver.
 
@@ -351,8 +360,9 @@ class DenseQPRegulator:
     def _reparameterize(self):
         """linearMPC.py:366-382: with an open-loop unstable A the reference optimises v in u = Krep x + v.
         ``A, Q, M, P, tq, G`` keep the reference's (v-space) meaning; the GPU solves the equivalent box QP
-        in u (``condense.input_space_operators``) and ``solve`` returns u, as the reference does after
-        mapping back (:507-509)."""
+        in u (``condense.input_space_operators``), or - where that QP is too ill-conditioned - the v-space
+        QP by interior point (``solver``), and ``solve`` returns u, as the reference does after mapping
+        back (:507-509)."""
         if np.any(np.abs(np.linalg.eigvals(self.A)) >= 1.0):
             self.A, self.Q, self.M = condense.reparameterize(self.A, self.B, self.Q, self.R, self.M, self.Krep)
             self.reparameterize = True
@@ -405,31 +415,48 @@ class DenseQPRegulator:
         rhs = (U - X0[:, :self._S.shape[1]] @ self._S.T).T
         return scipy.linalg.solve_triangular(self._T, rhs, lower=True, unit_diagonal=True).T
 
+    @property
+    def solver(self):
+        """Which GPU solver this regulator uses: "dr" - Douglas-Rachford on the (input-space) box QP, or "ipm" - the
+        interior-point method on the stagewise v-space QP (``csrc/ipm.cu``), taken by re-parameterised regulators
+        whose input-space Hessian the box path cannot use (its factorisation fails, it has non-finite entries, or its
+        condition number is 1e10 or more)."""
+        return self._solver
+
     def _setup_solver(self):
         n = self.N * self.Nu
         if n % 2:
             raise NotImplementedError("N*Nu must be even")
         P, tq = self._Pu, self._tqu
+        # A strongly unstable plant makes the input-space image of the v-space Hessian ill-conditioned (cond grows
+        # like rho^2N) or numerically indefinite; its QP is then solved in v by the interior-point kernel instead.
+        if self.reparameterize and not np.all(np.isfinite(P)):
+            return self._setup_ipm()
         # One-time dense linear algebra of the set-up (Cholesky of P, (P + D)^-1, extreme eigenvalues).  The reference
         # does its set-up with NumPy/SciPy on the host (:384-395); at n >= 4096 (CDU horizons x1/x2/x4: n = 4480 /
         # 8960 / 17920, 2 n^3 up to 1.2e13 flop) the same LAPACK-style calls run on the GPU through torch.linalg
         # (cuSOLVER, FP64) so that the set-up stays in seconds.  Library code at set-up time only - no solve goes
         # through it.
-        if n >= 4096 and os.environ.get("NNMPC_SETUP", "gpu") != "host":
-            self.Kunc, (lmin, lmax), self.rho_vec, Top, Mtq = self._setup_dense_gpu(P, tq)
-        else:
-            cho = scipy.linalg.cho_factor(P, lower=True)
-            self.Kunc = -scipy.linalg.cho_solve(cho, tq)                # unconstrained law u = Kunc x0
-            lmin, lmax = condense.extreme_eigs(P, cho)
-            self.rho_vec = self._penalty(P, lmin, lmax)
-            Minv = scipy.linalg.inv(P + np.diag(self.rho_vec))
-            Minv = 0.5 * (Minv + Minv.T)
-            Top, Mtq = Minv * self.rho_vec[None, :], Minv @ tq
+        try:
+            if n >= 4096 and os.environ.get("NNMPC_SETUP", "gpu") != "host":
+                self.Kunc, (lmin, lmax), self.rho_vec, Top, Mtq = self._setup_dense_gpu(P, tq)
+            else:
+                cho = scipy.linalg.cho_factor(P, lower=True)
+                self.Kunc = -scipy.linalg.cho_solve(cho, tq)                # unconstrained law u = Kunc x0
+                lmin, lmax = condense.extreme_eigs(P, cho)
+                self.rho_vec = self._penalty(P, lmin, lmax)
+                Minv = scipy.linalg.inv(P + np.diag(self.rho_vec))
+                Minv = 0.5 * (Minv + Minv.T)
+                Top, Mtq = Minv * self.rho_vec[None, :], Minv @ tq
+        except Exception as exc:
+            if self.reparameterize and _is_factorisation_error(exc):
+                return self._setup_ipm()
+            raise
         self.eig_range = (lmin, lmax)
         if self.reparameterize and not lmax / lmin < 1e10:
-            raise NotImplementedError(
-                f"re-parameterised regulator: the input-space Hessian has condition number {lmax / lmin:.1e}; plants this "
-                "unstable over the horizon need the v-space general-G splitting, which is not built (DESIGN.md)")
+            del Top, Mtq
+            return self._setup_ipm()
+        self._solver = "dr"
         self._nxa_ld = (self.Nx + 1) & ~1
 
         def pad(Mx):
@@ -448,6 +475,36 @@ class DenseQPRegulator:
         self._handle = hnd
         rho = _lib.host(self.rho_vec)
         _lib.check(L.nnmpc_qp_set_penalty(hnd, _lib.hptr(rho)), "nnmpc_qp_set_penalty")
+
+    def _setup_ipm(self):
+        """Interior-point regulator (nnmpc_qp_create_ipm) on the stagewise v-space QP of the re-parameterised plant:
+        stage weights ``Q, R, M`` (v-space, as held after ``_reparameterize``), dynamics ``A = A_open + B Krep``,
+        terminal weight ``Pf`` and bounds on ``u = Krep x + v``."""
+        nxa, nu = self.Nx, self.Nu
+        self._nxa_ld = (nxa + 1) & ~1
+        if self._nxa_ld > 64 or nu > 32:
+            raise NotImplementedError(
+                f"re-parameterised regulator with Nxa = {nxa}, Nu = {nu}: the input-space box QP is too ill-conditioned "
+                "for the Douglas-Rachford path, and the interior-point solver holds at most Nxa = 64 states (after "
+                "padding to an even count) and Nu = 32 inputs")
+        if not hasattr(self, "eig_range"):
+            self.eig_range = (float("nan"), float("nan"))
+        ld = self._nxa_ld
+
+        def pad(Mx, rows, cols):
+            out = np.zeros((rows, cols))
+            out[:Mx.shape[0], :Mx.shape[1]] = Mx
+            return out
+        ops = [pad(self.A, ld, ld), pad(self.B, ld, nu), pad(self.Q, ld, ld), _lib.host(self.R), pad(self.M, ld, nu),
+               pad(self.Pf, ld, ld), pad(self.Krep, nu, ld)]
+        L = _lib.lib()
+        hnd = C.c_void_p()
+        rc = L.nnmpc_qp_create_ipm(C.byref(hnd), ld, nu, self.N, *[_lib.hptr(a) for a in ops], self._dev)
+        _lib.check(rc, "nnmpc_qp_create_ipm")
+        self._handle = hnd
+        self._solver = "ipm"
+        if self.max_iter == DEFAULT_MAX_ITER:      # the Douglas-Rachford budget; an interior point needs tens
+            self.max_iter = IPM_MAX_ITER
 
     def _penalty(self, P, lmin, lmax):
         """ADMM penalty vector: 0.5 sqrt(lmin lmax) (swept on the CDU closed loop, 0.28 .. 1.1, B200 round 1ae) spread
